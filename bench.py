@@ -2,6 +2,7 @@
 """Benchmark of the NSGP-RePRE hot path (BASELINE.json metric, configs[1]).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path over one synthetic batch
@@ -319,6 +320,25 @@ def read_traffic():
         return {}
 
 
+def dump_outputs(out_dir, arrays, sample=1 << 17):
+    """Writes every (name, tensor) of `arrays` as out_dir/<name>.npy, float32 (integer tensors
+    as float64).  A tensor of more than `sample` elements is written as its elements at
+    `sample` flat indices drawn by numpy.random.default_rng(0) and sorted: the same positions
+    in every run and every build.  A step's dump stays within 64 MB."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in arrays:
+        t = t.detach()
+        if t.numel() > sample:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), sample, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        a = t.cpu().numpy().astype(np.float32 if t.is_floating_point() else np.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        total += a.nbytes
+    assert total <= 64 << 20, total
+
+
 # --------------------------------------------------------------------------- main
 def main():
     ap = argparse.ArgumentParser()
@@ -335,7 +355,14 @@ def main():
     ap.add_argument("--cpu-budget-s", type=float, default=15.0)
     ap.add_argument("--stage-sms", type=int, default=None,
                     help="SMs of the staging half of the pipelined covariance pass (0: serial)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy "
+                         "(see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     cfg = dict(CONFIGS[args.config])
     for k in ("batch", "height", "width"):
@@ -406,7 +433,6 @@ def main():
     from nsgp_repre_b200 import standin, _lib
     assert pkg._lib.engine() == 0
 
-    torch.backends.cudnn.benchmark = True         # stand-in detector only (e2e leg)
     torch.manual_seed(1234)
     model = standin.FasterRCNNStandIn(with_rpn=False, with_roi=False).to(dev).eval()
     layers = trace_layers(H, W, standin)
@@ -428,8 +454,13 @@ def main():
     cap = [m.register_forward_hook(
         lambda m, i, o: layer_inputs.__setitem__(names[m], i[0].detach().contiguous()))
         for m in model.modules() if isinstance(m, torch.nn.Conv2d)]
+    # deterministic cuDNN algorithms: the same arguments give the same layer inputs in every
+    # run, so that the outputs of two builds can be compared (--dump-outputs)
+    torch.backends.cudnn.deterministic = True
     with torch.no_grad():
         model(images_h.to(dev, non_blocking=True))
+    torch.backends.cudnn.deterministic = False
+    torch.backends.cudnn.benchmark = True         # stand-in detector only (e2e leg)
     for h in cap:
         h.remove()
     torch.cuda.synchronize()
@@ -496,10 +527,12 @@ def main():
         proto.build(f, l, range(C_OLD))
         return proto.staged()
 
+    last = {}
+
     def hot_step():
         # the three phases are independent; RePRE goes first because its host read would
         # otherwise wait behind the grouped covariance launches
-        repre_step(feats_d, labels_d)
+        last["replay_input"] = repre_step(feats_d, labels_d)
         cov_pass()
         sgd_step()
 
@@ -550,6 +583,14 @@ def main():
                                                      reduce_tail if world > 1 else None)
     clk = clocks.stop() if rank == 0 else None
     ms_per_step = total_ms / args.steps
+    if args.dump_outputs is not None and rank == 0:
+        # what a caller holds after the last timed step: the replay classifier input and its
+        # labels, the covariance sums (finalised) and the projected-SGD-updated weights
+        dump_outputs(args.dump_outputs,
+                     [("replay_input", last["replay_input"]),
+                      ("prototype_labels", proto.tmp_label)] +
+                     [("cov." + k, v) for k, v in sorted(hooks.fea_in.items())] +
+                     [("param." + n, p) for n, p in named])
     if os.environ.get("NSGP_TIMELINE") and _lib.HAS_BRINGUP and rank == 0:
         # developers only (bring-up library): kernel timeline of the last timed steps
         import ctypes

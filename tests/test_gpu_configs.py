@@ -500,7 +500,7 @@ def test_reference_config_keys_feed_the_dropins(pkg, tmp_path):
 
 
 # ------------------------------------------------------------------ N > 1 on NCCL
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 def test_two_gpu_job_reduces_and_shards_correctly():
     """torchrun x2 over NCCL: the timed job ends with the ONE all-reduce of the flat arena; the
     finalised covariance after the reduce equals the sum of the per-rank results

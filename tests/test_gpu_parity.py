@@ -854,15 +854,18 @@ def test_roi_extract_empty_and_errors(pkg):
 
 
 # ------------------------------------------------------------------------- bench contract
-def test_bench_line_contract():
-    """`python bench.py` prints ONE JSON line with the keys the driver reads (small run)."""
+def test_bench_line_contract(tmp_path):
+    """`python bench.py` prints ONE JSON line with the keys the driver reads (small run) and
+    writes the outputs of its last timed step under --dump-outputs."""
     import json
     import subprocess
     import sys
+    import numpy as np
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dump = tmp_path / "outputs"
     out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "2",
-                          "--warmup", "3", "--cpu-budget-s", "0.5"], capture_output=True,
-                         text=True, timeout=600, cwd=root)
+                          "--warmup", "3", "--cpu-budget-s", "0.5", "--dump-outputs", str(dump)],
+                         capture_output=True, text=True, timeout=600, cwd=root)
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [ln for ln in out.stdout.splitlines() if ln.strip()]
     assert len(lines) == 1
@@ -886,6 +889,16 @@ def test_bench_line_contract():
     assert set(("value", "unit", "h2d_bytes_per_step", "d2h_bytes_per_step")) <= set(d["e2e"])
     assert d["e2e"]["h2d_bytes_per_step"] > 3e8 and d["e2e"]["value"] < d["value"]
     assert d["gpu_launches"] > 0 and d["config"]["config_index"] == 1
+    arrays = {f[:-4]: np.load(str(dump / f)) for f in os.listdir(str(dump))}
+    assert all(f.endswith(".npy") for f in os.listdir(str(dump)))
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    assert len([k for k in arrays if k.startswith("cov.")]) == 61
+    assert len([k for k in arrays if k.startswith("param.")]) > 0
+    P = d["roofline_repre"]["prototypes"]
+    assert arrays["replay_input"].size == min(P * 256 * 7 * 7, 1 << 17)   # sampled above 2^17
+    assert arrays["prototype_labels"].shape == (P,)
+    assert all(np.isfinite(a).all() for a in arrays.values())
 
 
 def test_bench_reference_arm_loads_no_product_code():
