@@ -162,7 +162,7 @@ typedef struct {
   int kind;
   int n_problems[4], n_items[4];   /* [0] single-CTA kernel, [1] CTA-pair (cta_group::2) kernel,
                                       [2] sliding-window autocorrelation kernel,
-                                      [3] wide-tile (128 x 256) Gram kernel */
+                                      [3] reserved, always zero */
   size_t off_probs[4], off_items[4];
   size_t bytes;
 } nsgp_group_t;

@@ -96,7 +96,7 @@ class CovarianceHooks:
     main_stream_ms = 0.45
 
     def __init__(self, model: nn.Module, ignore_keys=(), add_default_ignores=True,
-                 mode="deferred", ring=3):
+                 mode="deferred"):
         """``mode``
         * ``"deferred"`` (default): a hook call only records its layer input; at the end of
           the forward (``flush``) ONE grouped staging launch (two when a gather layout needs
@@ -111,19 +111,16 @@ class CovarianceHooks:
           (``flush``) the Gram updates of all staged layers run as ONE persistent
           tcgen05 launch on a side stream, overlapping the next forward.  Two workspace
           sets alternate so the next forward never waits for the launch in flight.
-        * ``"overlap"``: per-layer launches, contraction of layer i on a side stream while
-          the caller's stream stages layer i+1; ``ring`` staged workspaces rotate.
-        * ``"immediate"``: stage + contract back to back on the caller's stream.
+        * ``"immediate"``: stage + contract back to back on the caller's stream, one layer
+          at a time.  The bring-up SIMT engine has no grouped launch and always runs this
+          way.
         Every result access joins the side stream first."""
         self.model = model
-        if mode not in ("deferred", "grouped", "overlap", "immediate"):
-            raise ValueError("mode must be 'deferred', 'grouped', 'overlap' or 'immediate'")
+        if mode not in ("deferred", "grouped", "immediate"):
+            raise ValueError("mode must be 'deferred', 'grouped' or 'immediate'")
         self.mode = mode
         self._sets = [_JobSet(), _JobSet()]
         self._cur = 0
-        self._ring_n = max(2, int(ring))
-        self._ring = []             # [workspace tensor, done event]
-        self._ring_pos = 0
         self._side = None
         self._pending = False
         self.ignore_keys = list(ignore_keys) + (self.DEFAULT_IGNORE if add_default_ignores else [])
@@ -202,23 +199,8 @@ class CovarianceHooks:
         if self._side is None or self._side.device != device:
             # high priority: the persistent contraction kernel gets its CTAs placed as soon
             # as blocks of the staging kernels (caller's stream) retire
-            import os
-            prio = -1 if os.environ.get("NSGP_SIDE_PRIO", "1") != "0" else 0
-            self._side = torch.cuda.Stream(device=device, priority=prio)
+            self._side = torch.cuda.Stream(device=device, priority=-1)
         return self._side
-
-    def _ring_slot(self, nbytes: int, device):
-        """Next staged workspace of the ring, grown on demand; the caller's stream
-        first waits until the contraction that last read it has finished."""
-        if len(self._ring) < self._ring_n:
-            self._ring.append([None, None])
-        slot = self._ring[self._ring_pos % len(self._ring)]
-        self._ring_pos += 1
-        if slot[1] is not None:
-            torch.cuda.current_stream(device).wait_event(slot[1])
-        if slot[0] is None or slot[0].numel() < nbytes or slot[0].device != device:
-            slot[0] = torch.empty(int(nbytes), dtype=torch.uint8, device=device)
-        return slot
 
     # ------------------------------------------------------------ grouped mode
     def _stage_job(self, x, key, geom, B, layout, la):
@@ -545,37 +527,14 @@ class CovarianceHooks:
             hit = ((Cin, H, W, kh, kw, sh, sw, ph, pw), B, layout, la)
             self._geom_cache[ck] = hit
         (Cin, H, W, kh, kw, sh, sw, ph, pw), B, layout, la = hit
-        mode = self.mode
-        if mode in ("grouped", "deferred") and _lib.engine() != 0:
-            mode = "overlap"            # the bring-up engine has no grouped launch
-        if mode in ("grouped", "deferred"):
+        # the bring-up engine has no grouped launch
+        if self.mode in ("grouped", "deferred") and _lib.engine() == 0:
             self._stage_job(x, key, (Cin, H, W, kh, kw, sh, sw, ph, pw), B, layout, la)
             return
-        if mode == "immediate":
-            ws = self._ws(layout.workspace_bytes, x.device)
-            check(lib.nsgp_cov_conv2d_accumulate(
-                ptr(x), B, Cin, H, W, kh, kw, sh, sw, ph, pw, ptr(la.acc), ptr(ws), ws.numel(),
-                _lib.current_stream(x.device)), "nsgp_cov_conv2d_accumulate")
-            la.calls += 1
-            return
-        # stage on the caller's stream (it produced x), contract on the side stream
-        slot = self._ring_slot(layout.workspace_bytes, x.device)
-        ws = slot[0]
-        main = torch.cuda.current_stream(x.device)
-        side = self._side_stream(x.device)
-        check(lib.nsgp_cov_conv2d_stage(
-            ptr(x), B, Cin, H, W, kh, kw, sh, sw, ph, pw, ptr(ws), ws.numel(),
-            main.cuda_stream), "nsgp_cov_conv2d_stage")
-        staged = torch.cuda.Event()
-        staged.record(main)
-        side.wait_event(staged)
-        check(lib.nsgp_cov_conv2d_contract(
-            Cin, H, W, kh, kw, sh, sw, ph, pw, ptr(la.acc), ptr(ws), ws.numel(),
-            side.cuda_stream), "nsgp_cov_conv2d_contract")
-        done = torch.cuda.Event()
-        done.record(side)
-        slot[1] = done
-        self._pending = True
+        ws = self._ws(layout.workspace_bytes, x.device)
+        check(lib.nsgp_cov_conv2d_accumulate(
+            ptr(x), B, Cin, H, W, kh, kw, sh, sw, ph, pw, ptr(la.acc), ptr(ws), ws.numel(),
+            _lib.current_stream(x.device)), "nsgp_cov_conv2d_accumulate")
         la.calls += 1
 
     def _accumulate_linear(self, x, key):

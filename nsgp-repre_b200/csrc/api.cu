@@ -174,7 +174,7 @@ int nsgp_cov_linear_layout(int d, nsgp_cov_layout_t* out) {
 static int cov_layers_group_build(const ConvGeom* geoms, float* const* stages, float* const* accs,
                                   int n, void* table_dev, size_t table_bytes, GroupInfo* gi,
                                   cudaStream_t stream) {
-  std::vector<ContractionArgs> probs, wide;
+  std::vector<ContractionArgs> probs;
   std::vector<ConvGeom> ac_g;
   std::vector<const float*> ac_s;
   std::vector<float*> ac_a;
@@ -187,30 +187,11 @@ static int cov_layers_group_build(const ConvGeom* geoms, float* const* stages, f
       ac_s.push_back(stages[i]);
       ac_a.push_back(accs[i]);
     }
-    for (int q = 0; q < np; ++q) {
-#ifdef NSGP_BRINGUP
-      if (gram_wide_eligible(p[q])) { wide.push_back(p[q]); continue; }   // NSGP_WIDE_KERNEL=1
-#endif
-      probs.push_back(p[q]);
-    }
+    probs.insert(probs.end(), p, p + np);
   }
   int rc = group_table_build(probs.data(), (int)probs.size(), kProfGram, table_dev, table_bytes,
                              gi, stream);
   if (rc) return rc;
-#ifdef NSGP_BRINGUP
-  if (!wide.empty()) {
-    const size_t off = (size_t)round_up((long long)gi->bytes, 256);
-    NSGP_REQUIRE(off <= table_bytes, "cov group: table too small");
-    SubGroup sg{};
-    rc = gram_wide_table_build(wide.data(), (int)wide.size(), (char*)table_dev + off,
-                               table_bytes - off, &sg, stream);
-    if (rc) return rc;
-    sg.off_probs += off;
-    sg.off_items += off;
-    gi->sub[3] = sg;
-    gi->bytes = sg.off_items + (size_t)sg.n_items * 32;
-  }
-#endif
   if (!ac_g.empty()) {
     const size_t off = (size_t)round_up((long long)gi->bytes, 256);
     NSGP_REQUIRE(off <= table_bytes, "cov group: table too small");
@@ -236,11 +217,7 @@ static size_t cov_layers_group_bytes(const ConvGeom* geoms, int n) {
     probs.insert(probs.end(), p, p + np);
     if (geoms[i].mode == kModeAutocorr && geoms[i].tiled) ac_g.push_back(geoms[i]);
   }
-  // eligible problems move to the wide table: bound both tables by the full list
   return group_table_bytes(probs.data(), (int)probs.size()) + 1024 +
-#ifdef NSGP_BRINGUP
-         gram_wide_table_bytes(probs.data(), (int)probs.size()) +
-#endif
          autocorr_table_bytes(ac_g.data(), (int)ac_g.size());
 }
 
@@ -394,9 +371,11 @@ static int sgd_tables(const nsgp_sgd_tensor_t* tensors, int n_tensors,
   return 0;
 }
 
+// slot [3] of nsgp_group_t is reserved and always zero
 static void group_to_abi(const GroupInfo& gi, nsgp_group_t* g) {
+  *g = nsgp_group_t{};
   g->kind = gi.kind;
-  for (int k = 0; k < 4; ++k) {
+  for (int k = 0; k < 3; ++k) {
     g->n_problems[k] = gi.sub[k].n_problems;
     g->n_items[k] = gi.sub[k].n_items;
     g->off_probs[k] = gi.sub[k].off_probs;
@@ -407,7 +386,7 @@ static void group_to_abi(const GroupInfo& gi, nsgp_group_t* g) {
 static GroupInfo group_from_abi(const nsgp_group_t& g) {
   GroupInfo gi{};
   gi.kind = g.kind;
-  for (int k = 0; k < 4; ++k)
+  for (int k = 0; k < 3; ++k)
     gi.sub[k] = SubGroup{g.n_problems[k], g.n_items[k], g.off_probs[k], g.off_items[k]};
   gi.bytes = g.bytes;
   return gi;
@@ -792,7 +771,7 @@ int nsgp_cov_pipeline_launch(const void* prev_table, const nsgp_group_t* prev_gr
   const GroupInfo gi = group_from_abi(*prev_group);
   const int ctas = sms - stage_sms;
   const bool have_ac = gi.sub[2].n_items > 0, have_gen = gi.sub[0].n_items > 0;
-  NSGP_REQUIRE(gi.sub[1].n_items == 0 && gi.sub[3].n_items == 0,
+  NSGP_REQUIRE(gi.sub[1].n_items == 0,
                "cov_pipeline_launch: bring-up sub-tables are not pipelined");
   // the staging half: the TMA kernel when the table has TMA items (the heavy routines), else
   // the register kernel's phase 0; whatever is left of phase 0 follows as an ordinary launch

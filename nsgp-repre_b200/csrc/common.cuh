@@ -101,11 +101,6 @@ struct Operand {
   int K;                   // valid columns
   int rows;                // valid virtual rows (<= T*Cs)
   long long tap_off[kMaxTaps];   // element offset of tap t (% 4 == 0)
-  int tile_nkb;            // > 0 (T == 1 only): tile-major storage - element (r, k) lives at
-                           // ((r/128) * tile_nkb + k/32) * 4096 + (r%128) * 32 + k%32, i.e. every
-                           // 128-row x 32-column TMA box is one contiguous 16 KB tile (TMA
-                           // sustains > 2x the bytes/cycle of 128 scattered 128-byte rows);
-                           // columns K .. 32*tile_nkb are stored as zeros
 };
 
 // Epilogue of the contraction engines.
@@ -135,8 +130,7 @@ struct SubGroup {
   size_t off_probs, off_items;
 };
 struct GroupInfo {
-  SubGroup sub[4];                 // [3] wide-tile Gram kernel (contraction_wide.cu),
-                                   // [0] single-CTA kernel, [1] CTA-pair kernel,
+  SubGroup sub[3];                 // [0] single-CTA kernel, [1] CTA-pair kernel,
                                    // [2] sliding-window autocorrelation kernel
   int kind;                        // ProfKind of the launches (kProfGram / kProfGemm)
   size_t bytes;
@@ -180,20 +174,12 @@ int autocorr_table_build(const ConvGeom* geoms, const float* const* stages, floa
 int autocorr_launch(const void* table_dev, const SubGroup& sg, cudaStream_t stream,
                     int max_ctas = 0, int pdl = 0);
 
-// wide-tile Gram kernel (contraction_wide.cu)
-struct ContractionArgs;
-bool gram_wide_eligible(const ContractionArgs& a);
-size_t gram_wide_table_bytes(const ContractionArgs* probs, int n);
-int gram_wide_table_build(const ContractionArgs* probs, int n, void* table_dev, size_t table_bytes,
-                          SubGroup* sg, cudaStream_t stream);
-int gram_wide_launch(const void* table_dev, const SubGroup& sg, cudaStream_t stream);
-
 // engines
 int contraction_simt(const ContractionArgs& a, cudaStream_t stream);
 int contraction_tc(const ContractionArgs& a, cudaStream_t stream);      // tcgen05/TMA
 int contraction(const ContractionArgs& a, cudaStream_t stream);         // dispatch on g_engine
 // One engine ships: tcgen05.  A -DNSGP_BRINGUP build (make BRINGUP=1) adds the SIMT
-// cross-check engine, the experiment kernels and the environment switches of DESIGN.md 6b.
+// cross-check engine, the CTA-pair kernel and the environment switches of DESIGN.md 6b.
 #ifdef NSGP_BRINGUP
 extern int g_engine;   // 0 = tcgen05 (product), 1 = SIMT (bring-up / cross-check)
 static inline const char* nsgp_env(const char* name) { return getenv(name); }

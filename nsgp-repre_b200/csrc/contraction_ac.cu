@@ -33,20 +33,13 @@ using namespace tc;
 
 namespace {
 
-constexpr int SA = 3;                       // A ring stages (upper bound; run-time value `sa`)
+constexpr int SA = 3;                       // A ring stages
 constexpr int SB = 4;                       // B ring stages (3 in the window + 1 in flight)
 constexpr uint32_t kPlane = BM * BK * 4;    // 16 KB: one hi or lo plane of a tile
 constexpr uint32_t kTile = 2 * kPlane;      // hi | lo
 // rows per work item = accumulation chain of 12 steps per row (bias of the truncating tensor-core
-// accumulate ~1.9e-8 per step); NSGP_AC_ROWS overrides for experiments
-static int rows_per_item() {
-  static const int v = [] {
-    const char* e = nsgp_env("NSGP_AC_ROWS");
-    const int r = e ? atoi(e) : 48;
-    return r >= 4 && r <= 256 ? r : 48;
-  }();
-  return v;
-}
+// accumulate ~1.9e-8 per step)
+constexpr int kRowsPerItem = 48;
 constexpr int kThreadsAc = 224;             // 7 warps: B producer, MMA, 4 epilogue, A producer
 constexpr size_t kSmemAc = (size_t)(SA + SB) * kTile + 1024 + 256;
 
@@ -89,14 +82,13 @@ __device__ unsigned long long g_ac_counters[160 * 8];
 
 __global__ void __launch_bounds__(kThreadsAc, 1)
 autocorr_tc_kernel(const AcProblem* __restrict__ probs, const AcItem* __restrict__ items,
-                   int n_items, int dbg, int sa_n, unsigned long long* tl,
-                   int wide_n, int tmem_a, int* __restrict__ sched) {
+                   int n_items, int dbg, unsigned long long* tl, int* __restrict__ sched) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>(
       (reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   uint8_t* a_ring = smem;                          // SA tiles
-  uint8_t* b_ring = smem + sa_n * kTile;           // SB tiles
-  uint64_t* a_full = reinterpret_cast<uint64_t*>(smem + (sa_n + SB) * kTile);
+  uint8_t* b_ring = smem + SA * kTile;             // SB tiles
+  uint64_t* a_full = reinterpret_cast<uint64_t*>(smem + (SA + SB) * kTile);
   uint64_t* a_empty = a_full + SA;
   uint64_t* b_full = a_empty + SA;
   uint64_t* b_empty = b_full + SB;
@@ -202,7 +194,7 @@ autocorr_tc_kernel(const AcProblem* __restrict__ probs, const AcItem* __restrict
       } else {
         const long long tile0 = ((long long)(sa * p.tiles + it.rb) * p.Hs + it.u0) * p.NS + st;
         for (int j = 0; j < n; ++j) {
-          const uint32_t s = cnt % sa_n, par = (cnt / sa_n) & 1;
+          const uint32_t s = cnt % SA, par = (cnt / SA) & 1;
           long long q0 = dbg ? clock64() : 0;
           mbar_wait_warp(&a_empty[s], par ^ 1, lane);
           if (dbg) c1 += clock64() - q0;
@@ -234,7 +226,7 @@ autocorr_tc_kernel(const AcProblem* __restrict__ probs, const AcItem* __restrict
       const uint32_t idesc = make_idesc_tf32(BM, (n_valid + 15) & ~15);
       // two accumulators at once need full 128-column tiles (the second starts at column 128)
       const uint32_t idesc2 = make_idesc_tf32(BM, 2 * BM);
-      const bool wide = wide_n != 0 && n_valid == BM;
+      const bool wide = n_valid == BM;
       const int n = it.u1 - it.u0;
       long long q0 = dbg ? clock64() : 0;
       mbar_wait_warp(tmem_empty, (n_done & 1) ^ 1, lane);     // epilogue drained the accumulators
@@ -246,7 +238,7 @@ autocorr_tc_kernel(const AcProblem* __restrict__ probs, const AcItem* __restrict
         mbar_wait_warp(&b_full[c % SB], (c / SB) & 1, lane);
       }
       for (int j = 0; j < n; ++j) {
-        const uint32_t as = a_cnt % sa_n, ap = (a_cnt / sa_n) & 1;
+        const uint32_t as = a_cnt % SA, ap = (a_cnt / SA) & 1;
         const uint32_t b2 = b_cnt + 2;
         long long q1 = dbg ? clock64() : 0;
         mbar_wait_warp(&a_full[as], ap, lane);
@@ -262,22 +254,6 @@ autocorr_tc_kernel(const AcProblem* __restrict__ probs, const AcItem* __restrict
         // shared-memory bandwidth (DESIGN.md 4).  Two neighbouring window tiles that are also
         // neighbours in the ring (no wrap) go through ONE N = 256 MMA into their two
         // neighbouring accumulators: A is read once for both.
-        if (tmem_a) {
-          // A from tensor memory: copy the A tile once (64 columns next to the accumulators,
-          // two buffers alternate), every MMA then reads only its B slice from shared memory
-          const uint32_t t_hi = tmem_base + 384 + (a_cnt & 1) * 64, t_lo = t_hi + 32;
-          tc_cp_a_kblock(t_hi, t_lo, a_hi, a_lo);
-          for (int dy = dy0; dy < 3;) {
-            const uint32_t bs = (b_cnt + dy) % SB;
-            const bool two = wide && dy + 1 < 3 && bs + 1 < SB;
-            const uint32_t bbase = smem_u32(b_ring + bs * kPlane);
-            tc_mma_kblock_3xtf32_ta(tmem_base + dy * BM, t_hi, t_lo,
-                                    make_kmajor_sw128_desc(bbase),
-                                    make_kmajor_sw128_desc(bbase + SB * kPlane),
-                                    two ? idesc2 : idesc, j > 0 ? 1u : 0u);
-            dy += two ? 2 : 1;
-          }
-        } else
         for (int dy = dy0; dy < 3;) {
           const uint32_t bs = (b_cnt + dy) % SB;
           const bool two = wide && dy + 1 < 3 && bs + 1 < SB;
@@ -413,7 +389,7 @@ size_t autocorr_table_bytes(const ConvGeom* geoms, int n) {
   for (int i = 0; i < n; ++i) {
     const ConvGeom& g = geoms[i];
     const size_t t = (size_t)ceil_div(g.C, BM);
-    items += 5 * t * t * (size_t)ceil_div(g.W, BK) * (size_t)ceil_div(g.H, rows_per_item());
+    items += 5 * t * t * (size_t)ceil_div(g.W, BK) * (size_t)ceil_div(g.H, kRowsPerItem);
   }
   return (size_t)n * sizeof(AcProblem) + items * sizeof(AcItem) + 1024;
 }
@@ -453,8 +429,8 @@ int autocorr_table_build(const ConvGeom* geoms, const float* const* stages, floa
       NSGP_REQUIRE(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled (autocorr) failed (%d)", (int)r);
     }
     const int strips = ceil_div(g.W, BK);
-    for (int u0 = 0; u0 < g.H; u0 += rows_per_item()) {
-      const int u1 = u0 + rows_per_item() < g.H ? u0 + rows_per_item() : g.H;
+    for (int u0 = 0; u0 < g.H; u0 += kRowsPerItem) {
+      const int u1 = u0 + kRowsPerItem < g.H ? u0 + kRowsPerItem : g.H;
       for (int st = 0; st < strips; ++st)
         for (int pass = 0; pass < 5; ++pass)
           for (int rb = 0; rb < p.tiles; ++rb)
@@ -501,22 +477,6 @@ int autocorr_table_build(const ConvGeom* geoms, const float* const* stages, floa
 int autocorr_launch(const void* table_dev, const SubGroup& sg, cudaStream_t stream, int max_ctas,
                     int pdl) {
   if (sg.n_items == 0) return 0;
-  // A-ring depth: 3 stages fill the SM; NSGP_AC_SA=2 (192 KB of ring) leaves ~34 KB for the
-  // L1 of co-resident staging kernels - measured equal end to end (scripts/overlap_probe.py:
-  // what the staging kernels lose next to this kernel is L1 capacity for loads in flight)
-  static const int sa_n = [] {
-    const char* e = nsgp_env("NSGP_AC_SA");
-    return (e && e[0] == '2') ? 2 : 3;
-  }();
-  static const int wide_n = [] {
-    const char* e = nsgp_env("NSGP_AC_WIDE");            // 0: three N = 128 MMAs per product
-    return (e && e[0] == '0') ? 0 : 1;
-  }();
-  static const int tmem_a = [] {
-    const char* e = nsgp_env("NSGP_AC_TMEMA");           // 1: A operand from tensor memory
-    return (e && e[0] == '1') ? 1 : 0;
-  }();
-  const size_t smem_bytes = (size_t)(sa_n + SB) * kTile + 1024 + 256;
   static bool configured = false;
   if (!configured) {
     NSGP_CHECK_CUDA(cudaFuncSetAttribute(autocorr_tc_kernel,
@@ -533,7 +493,7 @@ int autocorr_launch(const void* table_dev, const SubGroup& sg, cudaStream_t stre
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(grid);
   cfg.blockDim = dim3(kThreadsAc);
-  cfg.dynamicSmemBytes = smem_bytes;
+  cfg.dynamicSmemBytes = kSmemAc;
   cfg.stream = stream;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
@@ -542,8 +502,8 @@ int autocorr_launch(const void* table_dev, const SubGroup& sg, cudaStream_t stre
   cfg.numAttrs = pdl ? 1 : 0;
   int* sched = reinterpret_cast<int*>(const_cast<char*>((const char*)table_dev) + sg.off_items +
                                       (size_t)sg.n_items * sizeof(AcItem));
-  NSGP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, autocorr_tc_kernel, probs, items, sg.n_items, dbg, sa_n,
-                                     timeline_slot(10), wide_n, tmem_a, sched));
+  NSGP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, autocorr_tc_kernel, probs, items, sg.n_items, dbg,
+                                     timeline_slot(10), sched));
   NSGP_LAUNCHED();
   return 0;
 }

@@ -46,6 +46,8 @@ constexpr uint32_t kStageBytes = 4 * kABytes;   // A_hi | A_lo | B_hi | B_lo
 // of large addends is a third as long, and the small terms do not get truncated at
 // the scale of the large sum.  The epilogue adds them in fp32 (round-to-nearest).
 constexpr uint32_t kTmemCols = 512;
+// K blocks the L2 prefetch cursor of the producer runs ahead of its loads
+constexpr int kPrefetchDist = 8;
 
 // number of br-row TMA boxes covering [r0, r0+128) below `rows`
 __device__ __forceinline__ int seg_count(int r0, int rows, int br) {
@@ -113,7 +115,7 @@ template <bool PAIR>
 __global__ void __launch_bounds__(kThreads, 1)
 contraction_tc_kernel(const __grid_constant__ TcMaps pmaps, const __grid_constant__ TcParams pp,
                       const TcProblem* __restrict__ gprobs, const TcItem* __restrict__ gitems,
-                      int n_items_max, int prefetch_dist, int dbg,
+                      int n_items_max, int dbg,
                       unsigned long long* tl, const int* __restrict__ n_items_dev) {
   // the item count may live in device memory (work lists generated on the device)
   const int n_items = n_items_dev != nullptr ? min(n_items_max, __ldg(n_items_dev)) : n_items_max;
@@ -175,14 +177,14 @@ contraction_tc_kernel(const __grid_constant__ TcMaps pmaps, const __grid_constan
     // ============================ TMA producer ============================
     // The whole warp runs the loop with warp-uniform values; the single issuing thread
     // is elected inside each asm block (see tc_common.cuh).  A second cursor runs
-    // prefetch_dist K blocks ahead and pulls the operand rows into L2 - by exactly one
+    // kPrefetchDist K blocks ahead and pulls the operand rows into L2 - by exactly one
     // worker per row block (diagonal tile for Gram, first tile of the row / column for
     // GEMM) - so that the ring's load latency is an L2 hit, not a DRAM fill that every
     // CTA of the wave waits for together.
     uint32_t stage = 0, phase = 0;
     int pf_idx = worker, pf_kb = 0;
     Item pf_it{};
-    bool pf_live = prefetch_dist > 0 && pf_idx < n_items;
+    bool pf_live = pf_idx < n_items;
     if (pf_live) { pf_it = fetch_item(&pmaps, &pp, gprobs, gitems, pf_idx); pf_kb = pf_it.kb0; }
     auto prefetch_step = [&]() {
       if (!pf_live) return;
@@ -194,20 +196,16 @@ contraction_tc_kernel(const __grid_constant__ TcMaps pmaps, const __grid_constan
         const int r0 = pf_it.rb * TILE + rank * BM;
         for (int r = r0; r < r0 + BM && r < q.A.rows; r += q.A.br) {
           const int t = r / q.A.Cs, c = r - t * q.A.Cs;
-          const int px = q.A.tile_nkb ? 0 : kx;
-          const int py = q.A.tile_nkb ? (((c >> 7) * q.A.tile_nkb + pf_kb) << 7) + (c & 127) : c;
-          tma_prefetch_2d_elect(&pf_it.maps->a[0][t], px, py);
-          tma_prefetch_2d_elect(&pf_it.maps->a[1][t], px, py);
+          tma_prefetch_2d_elect(&pf_it.maps->a[0][t], kx, c);
+          tma_prefetch_2d_elect(&pf_it.maps->a[1][t], kx, c);
         }
       }
       if (pb) {
         const int c0 = pf_it.cb * TILE + rank * BM;
         for (int r = c0; r < c0 + BM && r < q.B.rows; r += q.B.br) {
           const int t = r / q.B.Cs, c = r - t * q.B.Cs;
-          const int px = q.B.tile_nkb ? 0 : kx;
-          const int py = q.B.tile_nkb ? (((c >> 7) * q.B.tile_nkb + pf_kb) << 7) + (c & 127) : c;
-          tma_prefetch_2d_elect(&pf_it.maps->b[0][t], px, py);
-          tma_prefetch_2d_elect(&pf_it.maps->b[1][t], px, py);
+          tma_prefetch_2d_elect(&pf_it.maps->b[0][t], kx, c);
+          tma_prefetch_2d_elect(&pf_it.maps->b[1][t], kx, c);
         }
       }
       if (++pf_kb >= pf_it.kb1) {
@@ -216,26 +214,24 @@ contraction_tc_kernel(const __grid_constant__ TcMaps pmaps, const __grid_constan
         if (pf_live) { pf_it = fetch_item(&pmaps, &pp, gprobs, gitems, pf_idx); pf_kb = pf_it.kb0; }
       }
     };
-    for (int i = 0; i < prefetch_dist; ++i) prefetch_step();
+    for (int i = 0; i < kPrefetchDist; ++i) prefetch_step();
     for (int idx = worker; idx < n_items; idx += n_workers) {
       const Item it = fetch_item(&pmaps, &pp, gprobs, gitems, idx);
       const TcParams& p = *it.p;
       const int r0 = it.rb * TILE + rank * BM;    // this CTA's A rows
       const int c0 = it.cb * TILE + rank * BM;    // the B rows this CTA stages
       const bool share = p.gram && p.same_operand && it.rb == it.cb;
-      const int a_rows = p.A.rows, a_br = p.A.br, a_cs = p.A.Cs, a_tn = p.A.tile_nkb;
-      const int b_rows = p.B.rows, b_br = p.B.br, b_cs = p.B.Cs, b_tn = p.B.tile_nkb;
+      const int a_rows = p.A.rows, a_br = p.A.br, a_cs = p.A.Cs;
+      const int b_rows = p.B.rows, b_br = p.B.br, b_cs = p.B.Cs;
       const int segs_a = seg_count(r0, a_rows, a_br);
       const int segs_b = share ? 0 : seg_count(c0, b_rows, b_br);
       // bytes landing on this CTA's full barrier per stage; full boxes always count
-      const uint32_t tx =
-          ((dbg & 4) ? 1u : 2u) * (uint32_t)(segs_a * a_br + segs_b * b_br) * BK * 4u;
+      const uint32_t tx = 2u * (uint32_t)(segs_a * a_br + segs_b * b_br) * BK * 4u;
       for (int kb = it.kb0; kb < it.kb1; ++kb) {
         prefetch_step();
-        long long t0 = (dbg & 1) ? clock64() : 0;
-        if (dbg & 8) mbar_wait(&empty_bar[stage], phase ^ 1);
-        else mbar_wait_warp(&empty_bar[stage], phase ^ 1, lane);
-        long long t1 = (dbg & 1) ? clock64() : 0;
+        long long t0 = dbg ? clock64() : 0;
+        mbar_wait_warp(&empty_bar[stage], phase ^ 1, lane);
+        long long t1 = dbg ? clock64() : 0;
         c_wait += t1 - t0;
         mbar_expect_tx_elect(&full_bar[stage], tx);
         const uint32_t sbase = smem_u32(smem + stage * kStageBytes);
@@ -244,25 +240,21 @@ contraction_tc_kernel(const __grid_constant__ TcMaps pmaps, const __grid_constan
           const int r = r0 + s * a_br;
           const int t = r / a_cs, c = r - t * a_cs;
           const uint32_t off = (uint32_t)(s * a_br) * (BK * 4);
-          const int lx = a_tn ? 0 : kx0;
-          const int ly = a_tn ? (((c >> 7) * a_tn + kb) << 7) + (c & 127) : c;
-          tma_load_2d_elect(sbase + off, &it.maps->a[0][t], &full_bar[stage], lx, ly);
-          if (!(dbg & 4)) tma_load_2d_elect(sbase + kABytes + off, &it.maps->a[1][t], &full_bar[stage], lx, ly);
+          tma_load_2d_elect(sbase + off, &it.maps->a[0][t], &full_bar[stage], kx0, c);
+          tma_load_2d_elect(sbase + kABytes + off, &it.maps->a[1][t], &full_bar[stage], kx0, c);
         }
         for (int s = 0; s < segs_b; ++s) {
           const int r = c0 + s * b_br;
           const int t = r / b_cs, c = r - t * b_cs;
           const uint32_t off = (uint32_t)(s * b_br) * (BK * 4);
-          const int lx = b_tn ? 0 : kx0;
-          const int ly = b_tn ? (((c >> 7) * b_tn + kb) << 7) + (c & 127) : c;
-          tma_load_2d_elect(sbase + 2 * kABytes + off, &it.maps->b[0][t], &full_bar[stage], lx, ly);
-          if (!(dbg & 4)) tma_load_2d_elect(sbase + 3 * kABytes + off, &it.maps->b[1][t], &full_bar[stage], lx, ly);
+          tma_load_2d_elect(sbase + 2 * kABytes + off, &it.maps->b[0][t], &full_bar[stage], kx0, c);
+          tma_load_2d_elect(sbase + 3 * kABytes + off, &it.maps->b[1][t], &full_bar[stage], kx0, c);
         }
-        if (dbg & 1) c_issue += clock64() - t1;
+        if (dbg) c_issue += clock64() - t1;
         if (++stage == STAGES) { stage = 0; phase ^= 1; }
       }
     }
-    if ((dbg & 1) && lane == 0) {
+    if (dbg && lane == 0) {
       g_dbg_counters[blockIdx.x * 8 + 3] = c_wait;
       g_dbg_counters[blockIdx.x * 8 + 4] = c_issue;
     }
@@ -282,19 +274,18 @@ contraction_tc_kernel(const __grid_constant__ TcMaps pmaps, const __grid_constan
                                     : make_idesc_tf32(BM, (n_valid + 15) & ~15);
         const uint32_t buf = local_item & 1;
         const uint32_t use = local_item >> 1;
-        long long ta = (dbg & 1) ? clock64() : 0;
+        long long ta = dbg ? clock64() : 0;
         mbar_wait_warp(&tmem_empty[buf], (use & 1) ^ 1, lane);   // epilogue drained this buffer
-        if (dbg & 1) c_acc += clock64() - ta;
+        if (dbg) c_acc += clock64() - ta;
         tc_fence_after();
         // single-CTA: [main | corr] x 128 columns per buffer; pair: one 256-column accumulator
         const uint32_t d_main = tmem_base + buf * 256;
         const uint32_t d_corr = d_main + 128;
         for (int kb = it.kb0; kb < it.kb1; ++kb) {
-          long long t0 = (dbg & 1) ? clock64() : 0;
-          if (dbg & 8) mbar_wait(&full_bar[stage], phase);
-          else mbar_wait_warp(&full_bar[stage], phase, lane);
+          long long t0 = dbg ? clock64() : 0;
+          mbar_wait_warp(&full_bar[stage], phase, lane);
           if (PAIR) mbar_wait_warp(&peer_full[stage], phase, lane);
-          long long t1 = (dbg & 1) ? clock64() : 0;
+          long long t1 = dbg ? clock64() : 0;
           c_wait += t1 - t0;
           ++c_kb;
           tc_fence_after();
@@ -309,12 +300,11 @@ contraction_tc_kernel(const __grid_constant__ TcMaps pmaps, const __grid_constan
             tc_commit_2sm_mc_elect(&empty_bar[stage]);        // frees the slot in both CTAs
             if (kb == it.kb1 - 1) tc_commit_2sm_mc_elect(&tmem_full[buf]);
           } else {
-            if (dbg & 2) tc_mma_kblock_3xtf32(d_main, d_corr, a_hi, a_hi, b_hi, b_hi, idesc, first, 2u);
-            else tc_mma_kblock_3xtf32(d_main, d_corr, a_hi, a_lo, b_hi, b_lo, idesc, first, 0u);
+            tc_mma_kblock_3xtf32(d_main, d_corr, a_hi, a_lo, b_hi, b_lo, idesc, first, 0u);
             tc_commit_elect(&empty_bar[stage]);               // slot free when these retire
             if (kb == it.kb1 - 1) tc_commit_elect(&tmem_full[buf]);
           }
-          if (dbg & 1) c_issue += clock64() - t1;
+          if (dbg) c_issue += clock64() - t1;
           if (++stage == STAGES) { stage = 0; phase ^= 1; }
         }
         if (it.kb1 <= it.kb0) {                               // defensive: empty K range
@@ -322,7 +312,7 @@ contraction_tc_kernel(const __grid_constant__ TcMaps pmaps, const __grid_constan
           else tc_commit_elect(&tmem_full[buf]);
         }
       }
-      if ((dbg & 1) && lane == 0) {
+      if (dbg && lane == 0) {
         g_dbg_counters[blockIdx.x * 8 + 0] = c_wait;
         g_dbg_counters[blockIdx.x * 8 + 1] = c_issue;
         g_dbg_counters[blockIdx.x * 8 + 2] = c_acc;
@@ -468,11 +458,6 @@ int encode_operand(const Operand& o, int br, CUtensorMap (*dst)[kMaxTaps]) {
                    "tcgen05 engine: operand base must be 16-byte aligned");
       cuuint64_t gdim[2] = {(cuuint64_t)o.K, (cuuint64_t)o.Cs};
       cuuint64_t gstr[1] = {(cuuint64_t)o.row_pitch * 4};
-      if (o.tile_nkb > 0) {            // tile-major: a (32, row blocks * K blocks * 128) matrix
-        gdim[0] = BK;
-        gdim[1] = (cuuint64_t)ceil_div(o.Cs, 128) * o.tile_nkb * 128;
-        gstr[0] = BK * 4;
-      }
       cuuint32_t box[2] = {(cuuint32_t)BK, (cuuint32_t)br};
       cuuint32_t estr[2] = {1, 1};
       CUresult r = enc(&dst[hl][t], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, (void*)base, gdim, gstr,
@@ -487,7 +472,6 @@ int encode_operand(const Operand& o, int br, CUtensorMap (*dst)[kMaxTaps]) {
 
 void fill_operand(const Operand& o, int br, TcOperand* d) {
   d->T = o.T; d->Cs = o.Cs; d->rows = o.rows; d->br = br;
-  d->tile_nkb = o.tile_nkb; d->pad0 = d->pad1 = d->pad2 = 0;
 }
 
 constexpr size_t kSmemBytes = (size_t)STAGES * kStageBytes + 1024 + 256;
@@ -496,17 +480,7 @@ constexpr size_t kSmemBytes = (size_t)STAGES * kStageBytes + 1024 + 256;
 constexpr size_t kSmemBytesFullSm = (size_t)7 * 32768 + 1024 + 256;
 
 int dbg_counters() {
-  static const int d = (nsgp_env("NSGP_DBG_COUNTERS") ? 1 : 0) | (nsgp_env("NSGP_DBG_MMA2") ? 2 : 0) |
-                       (nsgp_env("NSGP_DBG_HALFLOAD") ? 4 : 0) | (nsgp_env("NSGP_DBG_ALLPOLL") ? 8 : 0);
-  return d;
-}
-
-// K blocks the L2 prefetch cursor runs ahead of the loads (NSGP_PREFETCH overrides)
-int prefetch_distance() {
-  static const int d = [] {
-    const char* e = nsgp_env("NSGP_PREFETCH");
-    return e ? atoi(e) : 8;
-  }();
+  static const int d = nsgp_env("NSGP_DBG_COUNTERS") ? 1 : 0;
   return d;
 }
 
@@ -549,7 +523,7 @@ int launch_kernel(bool pair, const TcMaps& maps, const TcParams& p, const TcProb
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     NSGP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, contraction_tc_kernel<true>, maps, p, gprobs, gitems,
-                                       n_items, prefetch_distance(), dbg_counters(),
+                                       n_items, dbg_counters(),
                                        (unsigned long long*)nullptr, (const int*)nullptr));
     NSGP_LAUNCHED();
     return 0;
@@ -571,7 +545,7 @@ int launch_kernel(bool pair, const TcMaps& maps, const TcParams& p, const TcProb
     cfg.attrs = attr;
     cfg.numAttrs = pdl ? 1 : 0;
     NSGP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, contraction_tc_kernel<false>, maps, p, gprobs, gitems,
-                                       n_items, prefetch_distance(), dbg_counters(),
+                                       n_items, dbg_counters(),
                                        kind == kProfGram ? timeline_slot(0) : nullptr,
                                        n_items_dev));
   }
@@ -616,9 +590,6 @@ int build_problem(const ContractionArgs& a, bool pair, TcProblem* out) {
                "tcgen05 engine: row pitch must be 16-byte");
   NSGP_REQUIRE(ceil_div(a.A.K, BK) == ceil_div(a.B.K, BK),
                "contraction: operands disagree on K blocks");
-  NSGP_REQUIRE((a.A.tile_nkb == 0 || (a.A.T == 1 && a.A.tile_nkb == ceil_div(a.A.K, BK))) &&
-                   (a.B.tile_nkb == 0 || (a.B.T == 1 && a.B.tile_nkb == ceil_div(a.B.K, BK))),
-               "tcgen05 engine: tile-major operands are single-tap with tile_nkb = K blocks");
   const int br_a = pick_box_rows(a.A), br_b = pick_box_rows(a.B);
   NSGP_REQUIRE(br_a > 0 && br_b > 0, "tcgen05 engine: operand rows per tap must be >= 8 "
                "(multiple of 8 when taps > 1)");
@@ -643,11 +614,7 @@ int build_problem(const ContractionArgs& a, bool pair, TcProblem* out) {
   p.tiles_n = ceil_div(a.n_cols, tile);
   NSGP_REQUIRE(!p.gram || p.tiles_m == p.tiles_n, "Gram: operands must have the same rows");
   p.n_tiles = p.gram ? p.tiles_m * (p.tiles_m + 1) / 2 : p.tiles_m * p.tiles_n;
-  static const int vec_red = [] {
-    const char* e = nsgp_env("NSGP_VEC_RED");
-    return (e && e[0] == '0') ? 0 : 1;
-  }();
-  p.vec_red = (vec_red && a.ld % 4 == 0 && (reinterpret_cast<uintptr_t>(a.out) & 15) == 0) ? 1 : 0;
+  p.vec_red = (a.ld % 4 == 0 && (reinterpret_cast<uintptr_t>(a.out) & 15) == 0) ? 1 : 0;
   p.splits = 1;
   return 0;
 }
@@ -657,13 +624,9 @@ int build_problem(const ContractionArgs& a, bool pair, TcProblem* out) {
 // keeps hi*hi in its own accumulator (4 steps per K block), the pair kernel has one
 // accumulator for all three products (12 steps per K block).
 int chain_limit(const TcParams& p) {
-  static const int gram_chain = [] {
-    const char* e = nsgp_env("NSGP_CHAIN");             // bring-up override
-    return e ? atoi(e) : kChainGram;
-  }();
   if (p.chain > 0) return p.pair && p.chain > 32 ? 32 : p.chain;
   if (!p.gram) return kChainGemm;
-  return p.pair ? 32 : gram_chain;
+  return p.pair ? 32 : kChainGram;
 }
 
 }  // namespace
@@ -806,7 +769,6 @@ int group_table_build(const ContractionArgs* probs, int n, int kind, void* table
     off = (size_t)round_up((long long)(sg.off_items + items[k].size() * sizeof(TcItem)), 64);
   }
   info->sub[2] = SubGroup{0, 0, 0, 0};
-  info->sub[3] = SubGroup{0, 0, 0, 0};
   info->bytes = off;
   NSGP_REQUIRE(info->bytes <= table_bytes, "group_build: table too small (%zu < %zu)",
                table_bytes, info->bytes);
@@ -867,11 +829,6 @@ int group_launch(const void* table_dev, const GroupInfo& info, cudaStream_t stre
     int rc = launch_kernel(k == 1, dummy_maps, dummy, probs, items, sg.n_items, info.kind, stream);
     if (rc) return rc;
   }
-  int rc = 0;
-#ifdef NSGP_BRINGUP
-  rc = gram_wide_launch(table_dev, info.sub[3], stream);
-  if (rc) return rc;
-#endif
   // autocorrelation sub-table last: its long items fill the machine best once the small
   // problems are out of the way
   return autocorr_launch(table_dev, info.sub[2], stream);

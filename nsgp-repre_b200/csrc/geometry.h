@@ -54,21 +54,9 @@ struct ConvGeom {
                 // contiguous per (copy, channel block, row, column strip)) for the
                 // sliding-window kernel; TMA of contiguous tiles sustains > 2x the bytes/cycle
                 // of 128 scattered 128-byte rows (scripts/tma_probe.py)
-  int ftiled;   // flat / explicit (single-tap operands): staged tile-major, 128 rows x 32 columns
-                // = 16 KB contiguous per (row block, K block) (Operand::tile_nkb); K tail zeroed
   int d;        // true covariance dimension C*kh*kw
   int d_int;    // internal accumulator dimension (T*Cs)
 };
-
-static inline bool flat_tiled_enabled() {
-  static const bool on = [] {
-    // measured (scripts/bench_cov.py, NSGP_TIMELINE=1): correct, but the generic contraction
-    // launch takes 1.33 ms either way and staging gets 2 % slower -> opt-in
-    const char* e = nsgp_env("NSGP_FLAT_TILED");
-    return e && e[0] == '1';
-  }();
-  return on;
-}
 
 static inline int floor_div(int a, int b) {
   int q = a / b, r = a % b;
@@ -95,11 +83,7 @@ static inline int make_conv_geom(int C, int H, int W, int kh, int kw, int sh, in
     g.mode = kModeAutocorr;
     g.T = 9; g.Cs = C; g.ncopy = 3;
     g.Hs = H + 2;                                  // two zero rows below
-    static const int ws_align = [] {
-      const char* e = nsgp_env("NSGP_WS_ALIGN");      // bring-up: row pitch alignment (floats)
-      return e ? atoi(e) : 4;
-    }();
-    g.Ws = (int)round_up(W + 2, ws_align);         // >= two zero columns on the right
+    g.Ws = (int)round_up(W + 2, 4);                // >= two zero columns on the right
     g.Ht = 0;
     g.d_int = kAcMats * C;
     g.tiled = (g_engine == 0 && autocorr_kernel_enabled()) ? 1 : 0;
@@ -132,15 +116,8 @@ static inline int make_conv_geom(int C, int H, int W, int kh, int kw, int sh, in
     g.Ht = 0;
   }
   g.d_int = g.T * g.Cs;
-  g.ftiled = (g.mode != kModeImplicit && g_engine == 0 && flat_tiled_enabled()) ? 1 : 0;
   *out = g;
   return 0;
-}
-
-// tile-major single-tap operands (flat / explicit): K blocks per row, element offset
-static inline int ft_nkb(const ConvGeom& g) { return ceil_div((long long)g.Hout * g.Wout, 32); }
-static inline __host__ __device__ long long ft_off(int r, int k, int nkb) {
-  return ((long long)(r >> 7) * nkb + (k >> 5)) * 4096 + (long long)(r & 127) * 32 + (k & 31);
 }
 
 // autocorr extras: edge columns (2 sides x 3 row shifts, pitch Hc) and corner pixels
@@ -162,7 +139,6 @@ static inline long long ac_cornerbuf_off(const ConvGeom& g) {
 }
 static inline long long stage_hl_stride(const ConvGeom& g) {
   if (g.mode == kModeAutocorr) return round_up(ac_cornerbuf_off(g) + 16LL * g.C, 4);
-  if (g.ftiled) return (long long)ceil_div(g.Cs, 128) * ft_nkb(g) * 4096;
   return (long long)g.Cs * g.Hs * g.Ws * g.ncopy;
 }
 static inline size_t stage_bytes(const ConvGeom& g) {
@@ -194,7 +170,6 @@ static inline Operand conv_operand(const ConvGeom& g, const float* stage) {
     o.K = g.Hout * g.Wout;
     o.rows = (g.mode == kModeExplicit) ? g.d : g.Cs;
     o.tap_off[0] = 0;
-    if (g.ftiled) { o.tile_nkb = ft_nkb(g); o.row_pitch = 32; }
   }
   return o;
 }

@@ -105,19 +105,6 @@ stage_conv_body_t(const float* __restrict__ x, float* __restrict__ stage, const 
       }
       v[e] = acc;
     }
-    if (g.ftiled) {
-      // tile-major single-tap operand (flat mode: copy = r = 0): 4 columns of one tile row,
-      // and the zero K tail of the row's last K block from the thread that ends the row
-      const int nkb = (HWout + 31) >> 5;
-      float* o = stage + ft_off(c, x4 * 4, nkb);
-      split_store4(o, o + hl_stride, v[0], v[1], v[2], v[3]);
-      if (x4 == W4 - 1)
-        for (int k = (x4 + 1) * 4; k < nkb * 32; k += 4) {
-          float* z = stage + ft_off(c, k, nkb);
-          split_store4(z, z + hl_stride, 0.f, 0.f, 0.f, 0.f);
-        }
-      continue;
-    }
     float* o = stage + (((long long)copy * g.Cs + c) * g.Hs + r) * g.Ws + x4 * 4;
     split_store4(o, o + hl_stride, v[0], v[1], v[2], v[3]);
   }
@@ -145,14 +132,12 @@ stage_conv_kernel(const float* __restrict__ x, float* __restrict__ stage, ConvGe
 // ---------------------------------------------------------------------------
 // 1x1 stride-1 conv input with H*W % 4 == 0: the staged plane is the batch mean of
 // x itself.  One thread per float4.
-// K4 > 0: tile-major destination (geometry.h ftiled), K4 = float4 groups per row (H*W/4)
 template <int B_UNROLL>
 __device__ __forceinline__ void
 stage_flat_vec_body(const float* __restrict__ x, float* __restrict__ stage, long long n4,
                     int B, long long img, long long hl_stride, long long first, long long step,
-                    long long end, int K4 = 0) {
+                    long long end) {
   const float inv_div = (float)B;
-  const int nkb = (K4 * 4 + 31) >> 5;
   if (end > n4) end = n4;
   for (long long i = first; i < end; i += step) {
     const float* p = x + i * 4;
@@ -169,17 +154,6 @@ stage_flat_vec_body(const float* __restrict__ x, float* __restrict__ stage, long
       float4 v = ldg_stream4(p + (long long)b * img);
       s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
     }
-    if (K4 > 0) {
-      const int c = (int)(i / K4), k4 = (int)(i - (long long)c * K4);
-      float* o = stage + ft_off(c, k4 * 4, nkb);
-      split_store4(o, o + hl_stride, s.x / inv_div, s.y / inv_div, s.z / inv_div, s.w / inv_div);
-      if (k4 == K4 - 1)
-        for (int k = K4 * 4; k < nkb * 32; k += 4) {
-          float* z = stage + ft_off(c, k, nkb);
-          split_store4(z, z + hl_stride, 0.f, 0.f, 0.f, 0.f);
-        }
-      continue;
-    }
     split_store4(stage + i * 4, stage + i * 4 + hl_stride, s.x / inv_div, s.y / inv_div,
                  s.z / inv_div, s.w / inv_div);
   }
@@ -188,8 +162,8 @@ stage_flat_vec_body(const float* __restrict__ x, float* __restrict__ stage, long
 template <int B_UNROLL>
 __global__ void __launch_bounds__(256)
 stage_flat_vec_kernel(const float* __restrict__ x, float* __restrict__ stage, long long n4,
-                      int B, long long img, long long hl_stride, int K4) {
-  stage_flat_vec_body<B_UNROLL>(x, stage, n4, B, img, hl_stride, blockIdx.x * (long long)blockDim.x + threadIdx.x, (long long)gridDim.x * blockDim.x, n4, K4);
+                      int B, long long img, long long hl_stride) {
+  stage_flat_vec_body<B_UNROLL>(x, stage, n4, B, img, hl_stride, blockIdx.x * (long long)blockDim.x + threadIdx.x, (long long)gridDim.x * blockDim.x, n4);
 }
 
 // Batch mean of x (B, n) -> out (n), n % 4 == 0, 16-byte aligned: first pass of the
@@ -589,17 +563,6 @@ stage_conv_explicit_body_t(const float* __restrict__ x, float* __restrict__ stag
       v[e] = acc;
       if (++ox == g.Wout) { ox = 0; ++oy; }
     }
-    if (g.ftiled) {
-      const int nkb = (K + 31) >> 5;
-      float* o = stage + ft_off(row, k, nkb);
-      split_store4(o, o + hl_stride, v[0], v[1], v[2], v[3]);
-      if (k4 == W4 - 1)
-        for (int kz = k + 4; kz < nkb * 32; kz += 4) {
-          float* z = stage + ft_off(row, kz, nkb);
-          split_store4(z, z + hl_stride, 0.f, 0.f, 0.f, 0.f);
-        }
-      continue;
-    }
     float* o = stage + (long long)row * g.Ws + k;
     split_store4(o, o + hl_stride, v[0], v[1], v[2], v[3]);
   }
@@ -670,36 +633,8 @@ stage_conv_explicit_kernel(const float* __restrict__ x, float* __restrict__ stag
                            (long long)gridDim.x * blockDim.x, 1LL << 62);
 }
 
-// The staging kernels use no shared memory, but the persistent contraction kernels they
-// overlap with need the maximum carve-out: an SM only changes its L1/shared split when it
-// is idle, so a staging kernel with the default (L1-heavy) preference keeps the
-// contraction CTAs waiting until whole SMs drain.  Ask for the same split everywhere.
-static void stage_prefer_shared_carveout() {
-  static const bool once = [] {
-    // measured: slower on its own (5.6 -> 6.1 ms per covariance pass) and no better when
-    // overlapped (5.0 -> 5.2 ms), so it is opt-in
-    const char* e = nsgp_env("NSGP_STAGE_CARVEOUT");
-    if (!(e && e[0] == '1')) return true;
-    const int co = cudaSharedmemCarveoutMaxShared;
-#define NSGP_CARVE(k) cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, co)
-    NSGP_CARVE(stage_conv_kernel);
-    NSGP_CARVE(stage_flat_vec_kernel<8>);
-    NSGP_CARVE(batch_mean_vec_kernel<8>);
-    NSGP_CARVE(stage_3x3s1_vec_kernel<8>);
-    NSGP_CARVE(stage_autocorr_kernel);
-    NSGP_CARVE(stage_autocorr_vec_kernel<8>);
-    NSGP_CARVE(stage_autocorr_edges_kernel);
-    NSGP_CARVE(stage_conv_explicit_kernel);
-#undef NSGP_CARVE
-    cudaGetLastError();
-    return true;
-  }();
-  (void)once;
-}
-
 int launch_stage_conv(const float* x, float* stage, const ConvGeom& g, int B,
                       float* mean_scratch, cudaStream_t stream) {
-  stage_prefer_shared_carveout();
   long long total = (g.mode == kModeExplicit) ? (long long)g.Cs * g.Ws
                                               : (long long)g.Cs * g.Hs * g.Ws * g.ncopy;
   long long hl = stage_hl_stride(g);
@@ -749,8 +684,7 @@ int launch_stage_conv(const float* x, float* stage, const ConvGeom& g, int B,
     long long n4 = (long long)g.C * g.H * g.W / 4;
     int blocks = (int)((n4 + 255) / 256);
     if (blocks > 148 * 16) blocks = 148 * 16;
-    stage_flat_vec_kernel<8><<<blocks, 256, 0, stream>>>(x, stage, n4, B, img, hl,
-                                                        g.ftiled ? g.H * g.W / 4 : 0);
+    stage_flat_vec_kernel<8><<<blocks, 256, 0, stream>>>(x, stage, n4, B, img, hl);
   } else if (g.mode == kModeImplicit && g.kh == 3 && g.kw == 3 && g.sh == 1 && g.sw == 1 &&
              g.ph == 1 && g.pw == 1 && aligned && g.W % 4 == 0) {
     long long n = (long long)g.C * g.Hs * (g.W / 4);
@@ -815,8 +749,7 @@ stage_group_kernel(const StageJobDev* __restrict__ jobs, const StageItem* __rest
     const long long img = (long long)g.C * g.H * g.W;
     switch (it.kind) {
       case kStFlatVec:
-        stage_flat_vec_body<8>(x, j.stage, img / 4, Bx, img, j.hl, first, step, end,
-                               g.ftiled ? g.H * g.W / 4 : 0);
+        stage_flat_vec_body<8>(x, j.stage, img / 4, Bx, img, j.hl, first, step, end);
         break;
       case kStAcVec:
         stage_autocorr_vec_body<8>(x, j.stage, g.C, g.H, g.W, Bx, j.hl, g.tiled,
@@ -833,7 +766,7 @@ stage_group_kernel(const StageJobDev* __restrict__ jobs, const StageItem* __rest
         stage_conv_body(x, j.stage, g, Bx, j.hl, first, step, end);
         break;
       case kStExplicit:
-        if (g.Wout % 4 == 0 && !g.ftiled)           // items are row-aligned (plan_stage_job)
+        if (g.Wout % 4 == 0)                        // items are row-aligned (plan_stage_job)
           stage_conv_explicit_row_body(x, j.stage, g, Bx, j.hl, it.lo, threadIdx.x, blockDim.x,
                                        end);
         else
@@ -1328,11 +1261,7 @@ stage_tma_kernel(const StageJobDev* __restrict__ jobs, const StageItem* __restri
 // lists: [0] phase 0, register kernel; [1] phase 1 (after the batch means; also the light
 // phase-0 routines when the TMA kernel takes the heavy ones); [2] phase 0, TMA kernel
 static bool stage_tma_enabled(int B) {
-  static const bool off = [] {
-    const char* e = nsgp_env("NSGP_STAGE_TMA");     // bring-up switch
-    return e && e[0] == '0';
-  }();
-  return !off && tma_box_rows(B) > 0 && tma_ring_stages(B) >= kTmaGroups;
+  return tma_box_rows(B) > 0 && tma_ring_stages(B) >= kTmaGroups;
 }
 
 // role: 0 = plain; 1 = this flat 1x1 job also writes the stride-2 subsample of a sibling job
@@ -1345,13 +1274,8 @@ static void plan_stage_job(const ConvGeom& g, int job, int B, bool have_mean,
   const long long img = (long long)g.C * g.H * g.W;
   const bool aligned = img % 4 == 0;
   const bool tma = stage_tma_enabled(B);
-  const bool tma_job = tma && img % 256 == 0 && !g.ftiled;
-  static const int skip_kinds = [] {             // bring-up: time the phases without a routine
-    const char* e = nsgp_env("NSGP_STAGE_SKIP");
-    return e ? atoi(e) : 0;
-  }();
+  const bool tma_job = tma && img % 256 == 0;
   auto add = [&](int list, int kind, int from_mean, long long total, long long chunk) {
-    if (skip_kinds >> kind & 1) return;
     for (long long lo = 0; lo < total; lo += chunk) {
       ++counts[list];
       if (items) {
@@ -1416,7 +1340,7 @@ static void plan_stage_job(const ConvGeom& g, int job, int B, bool have_mean,
     for (int row = 0; row < g.Cs; ++row)
       for (long long lo = 0; lo < w4; lo += kVec) {
         ++counts[two ? 1 : light];
-        if (items && !(skip_kinds >> kStExplicit & 1)) {
+        if (items) {
           StageItem it{};
           it.job = job; it.kind = (short)kStExplicit; it.from_mean = (short)(two ? 1 : 0);
           it.lo = row * w4 + lo;
@@ -1436,10 +1360,9 @@ using tc::sm_count;
 // the TMA consumer that stages `full` writes it along (no second read of the input)
 static bool stage_sub_pair_ok(const ConvGeom& sub, const ConvGeom& full, int B) {
   const long long img = (long long)full.C * full.H * full.W;
-  return stage_tma_enabled(B) && img % 256 == 0 && full.W % 4 == 0 && !full.ftiled &&
-         !sub.ftiled && full.mode == kModeFlat && sub.mode == kModeFlat && full.sh == 1 &&
-         full.sw == 1 && sub.sh == 2 && sub.sw == 2 && sub.C == full.C && sub.H == full.H &&
-         sub.W == full.W && sub.Wout * 2 == full.W;
+  return stage_tma_enabled(B) && img % 256 == 0 && full.W % 4 == 0 && full.mode == kModeFlat &&
+         sub.mode == kModeFlat && full.sh == 1 && full.sw == 1 && sub.sh == 2 && sub.sw == 2 &&
+         sub.C == full.C && sub.H == full.H && sub.W == full.W && sub.Wout * 2 == full.W;
 }
 
 size_t stage_group_bytes(const ConvGeom* geoms, int n, int B) {
@@ -1627,30 +1550,17 @@ int stage_group_launch_tma(const void* table_dev, const StageGroupInfo& info, in
 // on the SMs the contraction grid left free; pdl: launched with the programmatic
 // stream-serialization attribute, i.e. it starts while the kernel queued before it is still
 // running.
-constexpr int kStagePartBlocksPerSm = 4;              // 256 threads x <= 64 registers
+// Blocks per SM: 4 x 256 threads x 64 registers fill the register file (the gather routines
+// are latency-bound: phase 1 0.58 -> 0.53 ms from 3 to 4 blocks; issuing the loads of two
+// positions per iteration was measured too: spills, 0.58 ms).
+constexpr int kStageBlocksPerSm = 4;
 constexpr size_t kStagePartSmem = 8 * 1024;
 int stage_group_launch_phase(const void* table_dev, const StageGroupInfo& info, int ph, int pdl,
                              int sms, cudaStream_t stream) {
   if (info.n_jobs == 0 || info.n_items[ph] == 0) return 0;
-  static const bool carve_once = [] {
-    const char* e = nsgp_env("NSGP_STAGE_GROUP_CARVEOUT");
-    const int co = e ? atoi(e) : -1;
-    if (co >= 0)
-      cudaFuncSetAttribute(stage_group_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, co);
-    return true;
-  }();
-  (void)carve_once;
   const char* t = (const char*)table_dev;
   ProfScope prof(kProfStage, stream);
-  // blocks per SM: 4 x 256 threads x 64 registers fill the register file (the gather
-  // routines are latency-bound: phase 1 0.58 -> 0.53 ms from 3 to 4 blocks; issuing the loads
-  // of two positions per iteration was measured too: spills, 0.58 ms)
-  static const int per_sm = [] {
-    const char* e = nsgp_env("NSGP_STAGE_BLOCKS_PER_SM");
-    const int v = e ? atoi(e) : 4;
-    return v > 0 && v <= 8 ? v : 4;
-  }();
-  int cap = sms > 0 ? sms * kStagePartBlocksPerSm : sm_count() * per_sm;
+  int cap = (sms > 0 ? sms : sm_count()) * kStageBlocksPerSm;
   int grid = info.n_items[ph] < cap ? info.n_items[ph] : cap;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(grid);

@@ -18,7 +18,7 @@ struct alignas(64) TcMaps {
 
 struct TcOperand {
   int T, Cs, rows, br;            // taps, rows per tap, valid rows, rows per TMA box
-  int tile_nkb, pad0, pad1, pad2; // > 0: tile-major storage (common.cuh Operand::tile_nkb)
+  int pad[4];
 };
 
 struct TcParams {
@@ -244,61 +244,6 @@ __device__ __forceinline__ void tc_mma_kblock_3xtf32(uint32_t d_main, uint32_t d
       "}" ::"r"(d_main),
       "r"(d_corr), "l"(a_hi), "l"(a_lo), "l"(b_hi), "l"(b_lo), "r"(idesc), "r"(first),
       "r"(same_acc)
-      : "memory");
-}
-
-// ---- A operand from tensor memory ------------------------------------------------
-// One K block of A (hi and lo planes, 128 rows x 32 fp32 each, K-major SWIZZLE_128B in shared
-// memory) copied into TMEM: 4 K steps x 8 columns per plane.  tcgen05.cp and tcgen05.mma
-// execute in issue order, so the MMAs that follow read the copied tile without a barrier.
-__device__ __forceinline__ void tc_cp_a_kblock(uint32_t t_hi, uint32_t t_lo, uint64_t a_hi,
-                                               uint64_t a_lo) {
-  asm volatile(
-      "{\n\t.reg .pred pe;\n\t.reg .b64 ah, al;\n\t"
-      "elect.sync _|pe, 0xffffffff;\n\t"
-      "@pe tcgen05.cp.cta_group::1.128x256b [%0], %2;\n\t"
-      "@pe tcgen05.cp.cta_group::1.128x256b [%1], %3;\n\t"
-      "add.u64 ah, %2, 2; add.u64 al, %3, 2;\n\t"
-      "@pe tcgen05.cp.cta_group::1.128x256b [%0 + 8], ah;\n\t"
-      "@pe tcgen05.cp.cta_group::1.128x256b [%1 + 8], al;\n\t"
-      "add.u64 ah, %2, 4; add.u64 al, %3, 4;\n\t"
-      "@pe tcgen05.cp.cta_group::1.128x256b [%0 + 16], ah;\n\t"
-      "@pe tcgen05.cp.cta_group::1.128x256b [%1 + 16], al;\n\t"
-      "add.u64 ah, %2, 6; add.u64 al, %3, 6;\n\t"
-      "@pe tcgen05.cp.cta_group::1.128x256b [%0 + 24], ah;\n\t"
-      "@pe tcgen05.cp.cta_group::1.128x256b [%1 + 24], al;\n\t"
-      "}" ::"r"(t_hi), "r"(t_lo), "l"(a_hi), "l"(a_lo)
-      : "memory");
-}
-// 3xTF32 K block with A read from TMEM (t_hi / t_lo as written by tc_cp_a_kblock), all three
-// products into one accumulator
-__device__ __forceinline__ void tc_mma_kblock_3xtf32_ta(uint32_t d, uint32_t t_hi, uint32_t t_lo,
-                                                        uint64_t b_hi, uint64_t b_lo,
-                                                        uint32_t idesc, uint32_t first) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred pe, pf, pt;\n\t"
-      ".reg .b64 bh, bl;\n\t"
-      "setp.eq.b32 pt, 0, 0;\n\t"
-      "elect.sync _|pe, 0xffffffff;\n\t"
-      "setp.ne.b32 pf, %6, 0;\n\t"
-      "@pe tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %3, %5, pf;\n\t"
-      "@pe tcgen05.mma.cta_group::1.kind::tf32 [%0], [%2], %3, %5, pt;\n\t"
-      "@pe tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %4, %5, pt;\n\t"
-      "add.u64 bh, %3, 2; add.u64 bl, %4, 2;\n\t"
-      "@pe tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1 + 8], bh, %5, pt;\n\t"
-      "@pe tcgen05.mma.cta_group::1.kind::tf32 [%0], [%2 + 8], bh, %5, pt;\n\t"
-      "@pe tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1 + 8], bl, %5, pt;\n\t"
-      "add.u64 bh, %3, 4; add.u64 bl, %4, 4;\n\t"
-      "@pe tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1 + 16], bh, %5, pt;\n\t"
-      "@pe tcgen05.mma.cta_group::1.kind::tf32 [%0], [%2 + 16], bh, %5, pt;\n\t"
-      "@pe tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1 + 16], bl, %5, pt;\n\t"
-      "add.u64 bh, %3, 6; add.u64 bl, %4, 6;\n\t"
-      "@pe tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1 + 24], bh, %5, pt;\n\t"
-      "@pe tcgen05.mma.cta_group::1.kind::tf32 [%0], [%2 + 24], bh, %5, pt;\n\t"
-      "@pe tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1 + 24], bl, %5, pt;\n\t"
-      "}" ::"r"(d),
-      "r"(t_hi), "r"(t_lo), "l"(b_hi), "l"(b_lo), "r"(idesc), "r"(first)
       : "memory");
 }
 

@@ -44,7 +44,7 @@ def run(mode, join_each):
           (mode, join_each, ms, host, flops / ms / 1e9, prof["gram"][0] / reps, prof["gram"][1] / reps,
            prof["stage"][0] / reps))
 
-modes = sys.argv[2].split(",") if len(sys.argv) > 2 else ("immediate", "overlap", "grouped")
+modes = sys.argv[2].split(",") if len(sys.argv) > 2 else ("immediate", "grouped", "deferred")
 def timeline():
     if not os.environ.get("NSGP_TIMELINE"):
         return
@@ -56,7 +56,7 @@ def timeline():
     ev = [(buf[2 * i], buf[2 * i + 1], kinds[i]) for i in range(m)]
     ev = ev[-int(os.environ.get('TL_N', '15')):]
     t0 = min(e[0] for e in ev)
-    names = {2: "stage", 0: "gram-generic", 10: "gram-autocorr", 11: "gram-wide"}
+    names = {2: "stage", 0: "gram-generic", 10: "gram-autocorr"}
     for a, b, k in sorted(ev):
         print("   %-14s %8.3f -> %8.3f ms  (%.3f)" % (names.get(k, k), (a - t0) / 1e6, (b - t0) / 1e6, (b - a) / 1e6))
 

@@ -41,6 +41,35 @@ def test_library_exports_every_header_symbol():
         assert s in pkg._lib.BRINGUP_SIGNATURES and not hasattr(pkg._lib.lib, s)
 
 
+def test_environment_switches_are_the_documented_ones():
+    """Every NSGP_* variable the bring-up library (nsgp_env) or the Python layer (os.environ)
+    reads is listed in DESIGN.md 6b, and every listed one is read.  NSGP_BRINGUP_LIB, which
+    selects the library, is described in the text above the table."""
+    pkg_dir = os.path.join(ROOT, "nsgp-repre_b200")
+    read = set()
+    csrc = os.path.join(pkg_dir, "csrc")
+    for name in os.listdir(csrc):
+        if not name.endswith((".cu", ".cuh", ".h")):
+            continue
+        with open(os.path.join(csrc, name), errors="replace") as f:
+            read |= set(re.findall(r'\bnsgp_env\(\s*"(NSGP_[A-Z0-9_]+)"', f.read()))
+    for name in os.listdir(pkg_dir):
+        if name.endswith(".py"):
+            with open(os.path.join(pkg_dir, name)) as f:
+                read |= set(re.findall(r'\bos\.environ(?:\.get\(|\[)\s*["\'](NSGP_[A-Z0-9_]+)',
+                                       f.read()))
+    read.discard("NSGP_BRINGUP_LIB")
+    design = open(os.path.join(ROOT, "DESIGN.md")).read()
+    section = re.search(r"^## 6b\..*?(?=^## )", design, flags=re.S | re.M)
+    assert section, "DESIGN.md lost section 6b"
+    documented = set()
+    for row in re.findall(r"^\|([^|\n]*)\|", section.group(0), flags=re.M):
+        documented |= set(re.findall(r"\bNSGP_[A-Z0-9_]+", row))
+    assert "NSGP_DBG_COUNTERS" in read
+    assert read == documented, "read, not documented: %s; documented, not read: %s" % (
+        sorted(read - documented), sorted(documented - read))
+
+
 def test_layout_queries_are_host_only():
     from nsgp_repre_b200._lib import lib, CovLayout
     L = CovLayout()
