@@ -924,8 +924,8 @@ int repre_segment_mean_dev(const float* F, int D, const int32_t* seg_offsets, co
 static void batched_layout(const int32_t* sizes, int n_classes, int D, size_t* n_total,
                            size_t* s_elems, size_t* table_bytes) {
   size_t n = 0, s = 0;
-  // the tcgen05 engine wants >= 8 operand rows: a smaller class is contracted as 8 rows
-  // (the extra rows are the next class's or padding; only its own n x n block is read back)
+  // a class of fewer than 8 rows is contracted as 8 rows (the extra rows are the next
+  // class's or padding; only its own n x n block is read back)
   for (int c = 0; c < n_classes; ++c) {
     const size_t ne = sizes[c] > 0 && sizes[c] < 8 ? 8 : (size_t)sizes[c];
     n += (size_t)sizes[c];

@@ -434,11 +434,17 @@ EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
+// Rows per TMA box.  A single-tap operand takes the largest power of two <= Cs (at most 128)
+// but never less than 8 rows, the 128-byte swizzle atom: box rows at or past Cs are out of
+// bounds, land in shared memory as zeros and are masked by the epilogue, so an operand of
+// 1..7 rows (a layer with 3 output channels, 3 kept-out directions, 5 centres) is one 8-row
+// box.  The rows of tap t > 0 start at t * Cs, so a multi-tap operand needs boxes that
+// divide Cs.
 int pick_box_rows(const Operand& o) {
   if (o.T == 1) {
     int br = 128;
-    while (br > o.Cs) br >>= 1;
-    return br < 8 ? 0 : br;
+    while (br > 8 && br > o.Cs) br >>= 1;
+    return br;
   }
   for (int br = 128; br >= 8; br >>= 1)
     if (o.Cs % br == 0) return br;
@@ -591,8 +597,8 @@ int build_problem(const ContractionArgs& a, bool pair, TcProblem* out) {
   NSGP_REQUIRE(ceil_div(a.A.K, BK) == ceil_div(a.B.K, BK),
                "contraction: operands disagree on K blocks");
   const int br_a = pick_box_rows(a.A), br_b = pick_box_rows(a.B);
-  NSGP_REQUIRE(br_a > 0 && br_b > 0, "tcgen05 engine: operand rows per tap must be >= 8 "
-               "(multiple of 8 when taps > 1)");
+  NSGP_REQUIRE(br_a > 0 && br_b > 0,
+               "tcgen05 engine: operand rows per tap must be a multiple of 8 when taps > 1");
   TcParams& p = out->p;
   p = TcParams{};
   p.nkb = k_blocks(a.A);

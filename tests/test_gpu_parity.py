@@ -571,8 +571,11 @@ def test_kmeans_assign_extension(pkg, engine):
     ws = torch.empty(lib.repre_kmeans_assign_workspace_bytes(n, k, D), dtype=torch.uint8,
                      device="cuda")
     lab = torch.empty(n, dtype=torch.int64, device="cuda")
-    pkg._lib.check(lib.repre_kmeans_assign(ptr(x.cuda()), n, D, ptr(cent.cuda()), k, ptr(lab),
-                                           ptr(ws), ws.numel(), _stream()), "kmeans")
+    # named, not temporaries: a freed temporary's memory can go to the next .cuda() copy
+    # before the kernel has read it
+    x_d, cent_d = x.cuda(), cent.cuda()
+    pkg._lib.check(lib.repre_kmeans_assign(ptr(x_d), n, D, ptr(cent_d), k, ptr(lab), ptr(ws),
+                                           ws.numel(), _stream()), "kmeans")
     want, _ = O.kmeans_assign(x.double(), cent.double())
     assert torch.equal(lab.cpu(), want)
 
