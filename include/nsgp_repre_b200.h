@@ -40,6 +40,19 @@ unsigned long long nsgp_launch_count(void);
  * kinds: 0 Gram contraction (tcgen05), 1 GEMM contraction (tcgen05), 2 staging,
  * 3 SGD prologue, 4 RePRE statistics.  nsgp_profile_read synchronises, returns the
  * summed milliseconds and launch count since the last read, and clears them. */
+/* Deterministic mode, process-wide (mirrors torch.use_deterministic_algorithms).  While it is
+ * set, size queries and table / plan builds produce work whose partial results meet in a fixed
+ * order: two launches with identical inputs give bitwise identical outputs on the same GPU model
+ * and library build, whatever the CTA count, SM partition or scheduling.  The size queries
+ * nsgp_cov_conv2d_layout (workspace_bytes), nsgp_cov_group_bytes, nsgp_sgd_plan_bytes,
+ * repre_build_prototypes_workspace_bytes, repre_cosine_count_batched_workspace_bytes and
+ * nsgp_ewc_table_bytes grow (partial-tile slots, fp64 partial sums).  A built table or plan
+ * keeps the mode it was built in.  Calls that have no deterministic form fail while it is set
+ * (nsgp_sgd_nscl_step and single-problem contractions that need a K split).  Returns the
+ * previous value. */
+int nsgp_set_deterministic(int on);
+int nsgp_get_deterministic(void);
+
 int nsgp_profile_enable(int on);
 int nsgp_profile_read(int kind, double* ms_total /* host */,
                       unsigned long long* launches /* host */);
@@ -162,7 +175,9 @@ typedef struct {
   int kind;
   int n_problems[4], n_items[4];   /* [0] single-CTA kernel, [1] CTA-pair (cta_group::2) kernel,
                                       [2] sliding-window autocorrelation kernel,
-                                      [3] reserved, always zero */
+                                      [3] ordered combine of a deterministic table: n_problems
+                                          partial-tile slots, n_items output tiles (zero when
+                                          built with nsgp_set_deterministic(0)) */
   size_t off_probs[4], off_items[4];
   size_t bytes;
 } nsgp_group_t;

@@ -73,6 +73,8 @@ SIGNATURES = {
     "nsgp_abi_version": (c_int, []),
     "nsgp_last_error": (C.c_char_p, []),
     "nsgp_launch_count": (C.c_ulonglong, []),
+    "nsgp_set_deterministic": (c_int, [c_int]),
+    "nsgp_get_deterministic": (c_int, []),
     "nsgp_profile_enable": (c_int, [c_int]),
     "nsgp_profile_read": (c_int, [c_int, C.POINTER(c_double), C.POINTER(C.c_ulonglong)]),
     "nsgp_cov_conv2d_layout": (c_int, [c_int] * 9 + [C.POINTER(CovLayout)]),
@@ -225,6 +227,34 @@ def current_stream(device=None) -> int:
 def require_cuda(t, name="tensor"):
     if not t.is_cuda:
         raise NsgpError("%s must live on a CUDA device (there is no CPU fallback)" % name)
+
+
+def deterministic() -> bool:
+    """Mirror ``torch.are_deterministic_algorithms_enabled()`` into the library (size queries and
+    table builds read it) and return it.  Called before every build or one-shot call; every cache
+    of a table, layout or plan has the returned mode in its key, so switching rebuilds."""
+    import torch
+    on = bool(torch.are_deterministic_algorithms_enabled())
+    lib.nsgp_set_deterministic(1 if on else 0)
+    return on
+
+
+def alert_not_deterministic(name: str) -> None:
+    """torch's contract for an operation without a deterministic implementation: raise
+    RuntimeError under ``torch.use_deterministic_algorithms(True)``, warn under
+    ``warn_only=True``, nothing when the switch is off."""
+    import torch
+    if not torch.are_deterministic_algorithms_enabled():
+        return
+    msg = ("%s does not have a deterministic implementation, but you set "
+           "'torch.use_deterministic_algorithms(True)'. You can turn off determinism just for this "
+           "operation, or you can use the 'warn_only=True' option, if that's acceptable for your "
+           "application." % name)
+    if torch.is_deterministic_algorithms_warn_only_enabled():
+        import warnings
+        warnings.warn(msg, UserWarning, stacklevel=3)
+    else:
+        raise RuntimeError(msg)
 
 
 PROFILE_KINDS = {"gram": 0, "gemm": 1, "stage": 2, "sgd": 3, "repre": 4}

@@ -60,6 +60,7 @@ class _JobSet:
         self.auto_sms = None    # ((rev, B), SMs of the staging half) chosen by _auto_stage_sms
         self.xs_arr = None      # reusable ctypes pointer table of the staging launch
         self.stage_jobs = None  # the CovJob array the staging table was built from
+        self.det = False        # deterministic mode the jobs and tables were built in
 
 
 class CovarianceHooks:
@@ -130,7 +131,8 @@ class CovarianceHooks:
         self._handles = []
         self._merged = {}           # key -> dense tensor added at finalize (old tasks)
         self._inflight = None       # deferred mode: the set staged but not yet contracted
-        self._geom_cache = {}       # (key, input shape, kernel, stride, padding) -> layout, layer
+        self._geom_cache = {}       # (key, input shape, kernel, stride, padding, device,
+                                    #  deterministic) -> layout, layer
         self._arena = None          # ONE flat fp32 buffer holding every planned accumulator
         self._alt = {}              # key -> _LayerAcc of the other layout kind (see _layer)
 
@@ -203,7 +205,7 @@ class CovarianceHooks:
         return self._side
 
     # ------------------------------------------------------------ grouped mode
-    def _stage_job(self, x, key, geom, B, layout, la):
+    def _stage_job(self, x, key, geom, B, layout, la, det):
         js = self._sets[self._cur]
         dev = x.device
         main = torch.cuda.current_stream(dev)
@@ -214,6 +216,12 @@ class CovarianceHooks:
             js.keep.clear()                   # ... and only then may its inputs be recycled
             js.xs = []
             js.versions = []
+            if js.det != det:
+                # workspaces and tables of the other deterministic mode: rebuild them all
+                del js.jobs[:]
+                js.sig = None
+                js.rev += 1
+                js.det = det
         # the same tensor with the same geometry earlier in this forward (e.g. the stage
         # output that feeds both layerN.0.conv1 and the FPN lateral conv): stage it once
         ident = (x.data_ptr(), x._version, tuple(x.shape), geom, B)
@@ -252,6 +260,8 @@ class CovarianceHooks:
             js.sig = None
             js.rev += 1
         js.seen.clear()
+        # the tables of this set are built in the mode its forward was recorded in
+        lib.nsgp_set_deterministic(1 if js.det else 0)
         dev = js.jobs[0][2].device
         main = torch.cuda.current_stream(dev)
         side = self._side_stream(dev)
@@ -512,8 +522,9 @@ class CovarianceHooks:
         if x.dtype != torch.float32 or not x.is_contiguous():
             x = x.float().contiguous()
         # layout + accumulator of (key, extent): looked up once, the hook runs per layer per
-        # forward on the training thread
-        ck = (key, x.shape, kernel_size, stride, padding, x.device)
+        # forward on the training thread.  The workspace size depends on the deterministic mode.
+        det = _lib.deterministic()
+        ck = (key, x.shape, kernel_size, stride, padding, x.device, det)
         hit = self._geom_cache.get(ck)
         if hit is None:
             B, Cin, H, W = x.shape
@@ -529,7 +540,7 @@ class CovarianceHooks:
         (Cin, H, W, kh, kw, sh, sw, ph, pw), B, layout, la = hit
         # the bring-up engine has no grouped launch
         if self.mode in ("grouped", "deferred") and _lib.engine() == 0:
-            self._stage_job(x, key, (Cin, H, W, kh, kw, sh, sw, ph, pw), B, layout, la)
+            self._stage_job(x, key, (Cin, H, W, kh, kw, sh, sw, ph, pw), B, layout, la, det)
             return
         ws = self._ws(layout.workspace_bytes, x.device)
         check(lib.nsgp_cov_conv2d_accumulate(

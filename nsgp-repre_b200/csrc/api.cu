@@ -18,6 +18,7 @@ int g_engine = 0;
 #endif
 
 int g_profile = 0;
+int g_deterministic = 0;
 namespace {
 struct ProfRec { cudaEvent_t a, b; };
 std::vector<ProfRec> g_prof[kProfKinds];
@@ -99,6 +100,13 @@ int nsgp_set_engine(int engine) {
 int nsgp_get_engine(void) { return g_engine; }
 #endif
 
+int nsgp_set_deterministic(int on) {
+  const int prev = g_deterministic;
+  g_deterministic = on ? 1 : 0;
+  return prev;
+}
+int nsgp_get_deterministic(void) { return g_deterministic; }
+
 int nsgp_profile_enable(int on) {
   int prev = g_profile;
   g_profile = on ? 1 : 0;
@@ -125,12 +133,15 @@ int nsgp_profile_read(int kind, double* ms_total, unsigned long long* launches) 
 // ---------------------------------------------------------------- covariance
 // Per-layer group table (autocorrelation layout: 29 problems -> one launch) kept behind
 // the staged operand in the same workspace.
+// Deterministic mode: every layer (not only the autocorrelation layout) contracts through such
+// a table, whose ordered combine needs its slots.
 static size_t layer_table_bytes(const ConvGeom& g) {
-  if (g.mode != kModeAutocorr) return 0;
+  if (g.mode != kModeAutocorr && !g_deterministic) return 0;
   ContractionArgs probs[kMaxConvProblems];
   int n = 0;
   conv_problems(g, nullptr, nullptr, probs, &n);
-  return group_table_bytes(probs, n) + 1024 + autocorr_table_bytes(&g, 1) + 256;
+  return group_table_bytes(probs, n) + 1024 +
+         (g.mode == kModeAutocorr ? autocorr_table_bytes(&g, 1) : 0) + 256;
 }
 
 int nsgp_cov_conv2d_layout(int C, int H, int W, int kh, int kw, int sh, int sw, int ph, int pw,
@@ -189,20 +200,36 @@ static int cov_layers_group_build(const ConvGeom* geoms, float* const* stages, f
     }
     probs.insert(probs.end(), p, p + np);
   }
+  // deterministic mode: one ordered combine for both kernels, grouped by output tile address
+  // (jobs of one module at several extents share an accumulator)
+  DetCombine det;
+  DetCombine* dp = g_deterministic ? &det : nullptr;
+  if (dp) {
+    group_table_count(probs.data(), (int)probs.size(), dp);
+    autocorr_count(ac_g.data(), ac_a.data(), (int)ac_g.size(), dp);
+  }
   int rc = group_table_build(probs.data(), (int)probs.size(), kProfGram, table_dev, table_bytes,
-                             gi, stream);
+                             gi, stream, dp);
   if (rc) return rc;
   if (!ac_g.empty()) {
     const size_t off = (size_t)round_up((long long)gi->bytes, 256);
     NSGP_REQUIRE(off <= table_bytes, "cov group: table too small");
     SubGroup sg{};
     rc = autocorr_table_build(ac_g.data(), ac_s.data(), ac_a.data(), (int)ac_g.size(),
-                              (char*)table_dev + off, table_bytes - off, &sg, stream);
+                              (char*)table_dev + off, table_bytes - off, &sg, stream, dp);
     if (rc) return rc;
     sg.off_probs += off;
     sg.off_items += off;
     gi->sub[2] = sg;
     gi->bytes = sg.off_items + (size_t)sg.n_items * 32 + 64;     // + the scheduler's counters
+  }
+  if (dp) {
+    const size_t end = det.layout(gi->bytes, &gi->sub[3]);
+    NSGP_REQUIRE(end <= table_bytes, "cov group: table too small for the ordered combine "
+                 "(%zu < %zu)", table_bytes, end);
+    gi->bytes = end;
+    rc = det_combine_upload(det, table_dev, gi->sub[3], stream);
+    if (rc) return rc;
   }
   return 0;
 }
@@ -264,8 +291,9 @@ int nsgp_cov_conv2d_contract(int C, int H, int W, int kh, int kw, int sh, int sw
   ContractionArgs probs[kMaxConvProblems];
   int n = 0;
   conv_problems(g, stage, acc, probs, &n);
-  if (n > 1 && g_engine == 0) {
-    // one or two persistent launches for all problems of the layer
+  if ((n > 1 || g_deterministic) && g_engine == 0) {
+    // one or two persistent launches for all problems of the layer (deterministic mode: always,
+    // the table orders the K-split partial tiles)
     char* table = align_up((char*)stage + stage_bytes(g), 256);
     const size_t room = (size_t)(((const char*)workspace + workspace_bytes) - table);
     GroupInfo gi{};
@@ -371,11 +399,12 @@ static int sgd_tables(const nsgp_sgd_tensor_t* tensors, int n_tensors,
   return 0;
 }
 
-// slot [3] of nsgp_group_t is reserved and always zero
+// slot [3] of nsgp_group_t describes the ordered combine of a deterministic table (zero
+// otherwise): n_problems slots at off_probs, n_items output tiles at off_items
 static void group_to_abi(const GroupInfo& gi, nsgp_group_t* g) {
   *g = nsgp_group_t{};
   g->kind = gi.kind;
-  for (int k = 0; k < 3; ++k) {
+  for (int k = 0; k < 4; ++k) {
     g->n_problems[k] = gi.sub[k].n_problems;
     g->n_items[k] = gi.sub[k].n_items;
     g->off_probs[k] = gi.sub[k].off_probs;
@@ -386,7 +415,7 @@ static void group_to_abi(const GroupInfo& gi, nsgp_group_t* g) {
 static GroupInfo group_from_abi(const nsgp_group_t& g) {
   GroupInfo gi{};
   gi.kind = g.kind;
-  for (int k = 0; k < 3; ++k)
+  for (int k = 0; k < 4; ++k)
     gi.sub[k] = SubGroup{g.n_problems[k], g.n_items[k], g.off_probs[k], g.off_items[k]};
   gi.bytes = g.bytes;
   return gi;
@@ -793,7 +822,10 @@ int nsgp_cov_pipeline_launch(const void* prev_table, const nsgp_group_t* prev_gr
     rc = stage_group_launch_phase(stage_table, si, 0, 0, 0, stream);
   }
   if (rc) return rc;
-  return stage_group_launch_phase(stage_table, si, 1, 0, 0, stream);
+  rc = stage_group_launch_phase(stage_table, si, 1, 0, 0, stream);
+  if (rc) return rc;
+  // deterministic table: the ordered combine of the contraction's partial tiles
+  return det_combine_launch(prev_table, gi.sub[3], gi.kind, stream);
 }
 
 // ---------------------------------------------------------------- RePRE
@@ -1023,8 +1055,8 @@ int repre_cosine_count_batched(const float* F, int D, const int32_t* rows, const
 namespace {
 struct ReBuildLayout {
   size_t off_hi, off_lo, off_S, off_prob, off_items, off_pairs, off_ext, off_cls, off_hdr,
-      off_nsaved, off_savedlen, off_greedy, bytes;
-  int ld_s, max_items, max_pairs;
+      off_nsaved, off_savedlen, off_greedy, off_slots, bytes;
+  int ld_s, max_items, max_pairs, det_slots;
 };
 ReBuildLayout rebuild_layout(int M, int D, int n_classes, int max_picks) {
   ReBuildLayout L{};
@@ -1049,6 +1081,10 @@ ReBuildLayout rebuild_layout(int M, int D, int n_classes, int max_picks) {
   L.off_savedlen = take((size_t)n_classes * 4);
   // greedy scratch: order (M ints), segment sizes / bases, covered flags (M bytes)
   L.off_greedy = take((size_t)M * 4 + (size_t)n_classes * (max_picks + 2) * 4 + (size_t)M + 256);
+  // deterministic mode: one partial-tile slot per work item when the Gram needs K splits
+  const int det_splits = ceil_div(ceil_div(D, 32), 64);   // K blocks per chain (tc::kChainGram)
+  L.det_slots = g_deterministic && det_splits > 1;
+  L.off_slots = take(L.det_slots ? (size_t)L.max_pairs * det_splits * kSlotElems * 4 : 0);
   L.bytes = off + 1024;
   return L;
 }
@@ -1120,14 +1156,19 @@ int repre_build_prototypes(const float* F, int D, int M, const int32_t* rows,
   const int nkb = ceil_div(D, 32);
   rc = launch_repre_plan(offsets, class_first, n_classes, L.ld_s, nsaved_dev, savedlen_dev, nkb,
                          L.max_items, ext, cls, ws + L.off_pairs, ws + L.off_items,
-                         ws + L.off_prob, hdr, stream);
+                         ws + L.off_prob, hdr, g_deterministic, stream);
   if (rc) return rc;
   rc = launch_repre_prepare(F, D, M, rows, offsets, class_first, hdr, hi, lo, ws + L.off_pairs, S,
                             L.ld_s, stream);
   if (rc) return rc;
+  float* slots = L.det_slots ? reinterpret_cast<float*>(ws + L.off_slots) : nullptr;
   rc = contraction_launch_dev_items(ws + L.off_prob, ws + L.off_items, L.max_items, hdr + 2,
-                                    kProfRepre, stream);
+                                    kProfRepre, slots, stream);
   if (rc) return rc;
+  if (slots != nullptr) {
+    rc = launch_repre_combine(ws + L.off_pairs, hdr, slots, S, L.ld_s, stream);
+    if (rc) return rc;
+  }
   rc = launch_threshold_count_dev(S, ext, n_classes, M, hdr, thresh, masks, counts, stream);
   if (rc) return rc;
   // density ordering + greedy cover + segment table + segment rows (one CTA per class)

@@ -88,6 +88,58 @@ ewc_penalty_kernel(const EwcTensorDev* __restrict__ tensors, int n, float coeff,
   }
 }
 
+// Deterministic mode: kEwcDetCtas CTAs stride over the chunks in a fixed order and write one
+// fp64 partial each behind the tensor table; one CTA sums them in a fixed order.
+constexpr int kEwcDetCtas = 512;
+
+__global__ void __launch_bounds__(256)
+ewc_penalty_partial_kernel(const EwcTensorDev* __restrict__ tensors, int n, int total_chunks,
+                           double* __restrict__ partial) {
+  double acc = 0.0;
+  for (int chunk = blockIdx.x; chunk < total_chunks; chunk += gridDim.x) {
+    const EwcTensorDev t = tensors[ewc_find(tensors, n, chunk)];
+    const long long beg = (long long)(chunk - t.chunk0) * kEwcChunk;
+    const long long end = min(t.numel, beg + kEwcChunk);
+    for (long long i = beg + threadIdx.x; i < end; i += 256) {
+      const float p = t.p[i];
+      for (int k = 0; k < t.tasks; ++k) {
+        const float d = p - t.old[(long long)k * t.numel + i];
+        const float w = t.imp[(long long)k * t.numel + i];
+        acc += (double)w * (double)d * (double)d;
+      }
+    }
+  }
+  __shared__ double red[8];
+  for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = acc;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double s = 0.0;
+    for (int w = 0; w < 8; ++w) s += red[w];
+    partial[blockIdx.x] = s;
+  }
+}
+
+__global__ void __launch_bounds__(256)
+ewc_penalty_sum_kernel(const double* __restrict__ partial, int n_partial, float coeff,
+                       double* __restrict__ loss) {
+  double acc = 0.0;
+  for (int i = threadIdx.x; i < n_partial; i += 256) acc += partial[i];
+  __shared__ double red[8];
+  for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = acc;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double s = 0.0;
+    for (int w = 0; w < 8; ++w) s += red[w];
+    *loss = (double)coeff * s;
+  }
+}
+
+static size_t ewc_tensors_bytes(int n) {
+  return (size_t)round_up((long long)(n > 0 ? n : 1) * sizeof(EwcTensorDev), 256);
+}
+
 static int ewc_table(const nsgp_ewc_tensor_t* tensors, int n, void* table_dev, size_t table_bytes,
                      cudaStream_t stream, int* total_chunks) {
   NSGP_REQUIRE(tensors && table_dev && n > 0, "ewc: bad arguments");
@@ -221,6 +273,19 @@ int nsgp_ewc_penalty(const nsgp_ewc_tensor_t* tensors, int n, float coeff, doubl
   for (int i = 0; i < n; ++i)
     NSGP_REQUIRE(tensors[i].p && (tensors[i].tasks == 0 || (tensors[i].importance && tensors[i].old_params)),
                  "ewc_penalty: tensor %d: null pointer", i);
+  if (g_deterministic) {
+    NSGP_REQUIRE(table_bytes >= ewc_tensors_bytes(n) + kEwcDetCtas * sizeof(double),
+                 "ewc_penalty: table too small for the deterministic sum (%zu < %zu)",
+                 table_bytes, ewc_tensors_bytes(n) + kEwcDetCtas * sizeof(double));
+    double* partial = reinterpret_cast<double*>((char*)table_dev + ewc_tensors_bytes(n));
+    const int ctas = chunks < kEwcDetCtas ? chunks : kEwcDetCtas;
+    ewc_penalty_partial_kernel<<<ctas, 256, 0, stream>>>(
+        reinterpret_cast<const EwcTensorDev*>(table_dev), n, chunks, partial);
+    NSGP_LAUNCHED();
+    ewc_penalty_sum_kernel<<<1, 256, 0, stream>>>(partial, ctas, coeff, loss_dev);
+    NSGP_LAUNCHED();
+    return 0;
+  }
   ewc_penalty_kernel<0><<<chunks, 256, 0, stream>>>(
       reinterpret_cast<const EwcTensorDev*>(table_dev), n, coeff, loss_dev, nullptr);
   NSGP_LAUNCHED();
@@ -244,7 +309,11 @@ int nsgp_ewc_penalty_backward(const nsgp_ewc_tensor_t* tensors, int n, float coe
   return 0;
 }
 
-size_t nsgp_ewc_table_bytes(int n) { return (size_t)(n > 0 ? n : 1) * sizeof(EwcTensorDev); }
+size_t nsgp_ewc_table_bytes(int n) {
+  // deterministic mode: + the fp64 partial sums of the penalty
+  if (g_deterministic) return ewc_tensors_bytes(n) + kEwcDetCtas * sizeof(double);
+  return (size_t)(n > 0 ? n : 1) * sizeof(EwcTensorDev);
+}
 
 int nsgp_pseudo_label_merge(const float* gt_boxes, const int32_t* gt_offsets,
                             const float* pseudo_boxes, const float* pseudo_scores,

@@ -6,6 +6,8 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <unordered_map>
+#include <vector>
 
 namespace nsgp {
 
@@ -36,6 +38,11 @@ extern unsigned long long g_launches;   // kernels launched by this library
     ++nsgp::g_launches;                                                           \
     NSGP_CHECK_CUDA(cudaGetLastError());                                          \
   } while (0)
+
+// ---- deterministic mode (nsgp_set_deterministic) -------------------------------
+// Size queries and table builds read it; a built table carries its mode in its work items,
+// so launching it never depends on the flag.
+extern int g_deterministic;
 
 // ---- optional per-kernel-kind device timing (bench.py's roofline leg) --------
 // When enabled every launch of a profiled kind is bracketed by a cudaEvent pair on
@@ -130,14 +137,61 @@ struct SubGroup {
   size_t off_probs, off_items;
 };
 struct GroupInfo {
-  SubGroup sub[3];                 // [0] single-CTA kernel, [1] CTA-pair kernel,
-                                   // [2] sliding-window autocorrelation kernel
+  SubGroup sub[4];                 // [0] single-CTA kernel, [1] CTA-pair kernel,
+                                   // [2] sliding-window autocorrelation kernel,
+                                   // [3] ordered combine (deterministic mode): n_problems =
+                                   //     partial-tile slots at off_probs, n_items = output
+                                   //     tiles (CombTile) at off_items
   int kind;                        // ProfKind of the launches (kProfGram / kProfGemm)
   size_t bytes;
 };
+
+// ---- ordered combine of partial tiles (deterministic mode) -------------------------
+// A work item whose output tile has other contributors in the same launch stores its fp32
+// partial tile (128 x 128, row-major, alpha applied, zeros where the epilogue masks) to a
+// slot instead of red.add'ing it; one short launch after the contraction then adds each
+// tile's slots into the running sum in slot order.  Slots are numbered by the table build,
+// so the result does not depend on which CTA ran which item or when.
+constexpr int kSlotElems = 128 * 128;
+struct alignas(16) CombTile {
+  float* out;              // first element of the output tile
+  int ld, rows, cols;      // leading dimension, valid rows / columns of the tile
+  int n, first;            // slot ids: list[first .. first + n), in summation order
+  int pad[2];
+};
+// Host side: count every (output tile, contributor) of a launch first, then assign.  A tile
+// with one contributor keeps the plain red.add (a single addend is exact and order-free).
+struct DetCombine {
+  std::unordered_map<const float*, int> counts;     // tile address -> contributors
+  std::unordered_map<const float*, int> tile_of;    // tile address -> index into tiles
+  std::vector<CombTile> tiles;
+  std::vector<std::vector<int>> per_tile;           // slot ids, in build order
+  int n_slots = 0;
+  void count(const float* tile) { ++counts[tile]; }
+  int contributors(const float* tile) const {
+    auto it = counts.find(tile);
+    return it == counts.end() ? 0 : it->second;
+  }
+  // slot id of one contribution to `tile`
+  int assign(float* tile, int ld, int rows, int cols);
+  // table memory from `off` on: CombTile[n] | int list | 256-aligned slots; fills sg and
+  // returns the end offset
+  size_t layout(size_t off, SubGroup* sg) const;
+  static size_t bytes_bound(size_t items) {
+    return items * ((size_t)kSlotElems * 4 + sizeof(CombTile) + 4) + 1024;
+  }
+};
+int det_combine_upload(const DetCombine& det, void* table_dev, const SubGroup& sg,
+                       cudaStream_t stream);
+int det_combine_launch(const void* table_dev, const SubGroup& sg, int kind, cudaStream_t stream);
+
 size_t group_table_bytes(const ContractionArgs* probs, int n);
+// det != nullptr: the caller counted every contribution of the launch into det (and lays
+// the combine out itself); det == nullptr in deterministic mode: the build does both
+void group_table_count(const ContractionArgs* probs, int n, DetCombine* det);
 int group_table_build(const ContractionArgs* probs, int n, int kind, void* table_dev,
-                      size_t table_bytes, GroupInfo* info, cudaStream_t stream);
+                      size_t table_bytes, GroupInfo* info, cudaStream_t stream,
+                      DetCombine* det = nullptr);
 int group_launch(const void* table_dev, const GroupInfo& info, cudaStream_t stream);
 // one sub-table of a group (0 generic kernel, 2 sliding-window kernel) on at most max_ctas
 // SMs (0: all); pdl: programmatic dependent launch behind the kernel queued before it;
@@ -145,8 +199,10 @@ int group_launch(const void* table_dev, const GroupInfo& info, cudaStream_t stre
 int group_launch_sub(const void* table_dev, const GroupInfo& info, int which, int max_ctas,
                      int pdl, cudaStream_t stream);
 
+// slots: partial tiles of the items that carry a slot id (deterministic mode), else NULL
 int contraction_launch_dev_items(const void* prob_dev, const void* items_dev, int max_items,
-                                 const int* n_items_dev, int kind, cudaStream_t stream);
+                                 const int* n_items_dev, int kind, float* slots,
+                                 cudaStream_t stream);
 int contraction_build_problem(const ContractionArgs& a, void* prob_host);
 size_t contraction_problem_bytes();
 size_t contraction_item_bytes();
@@ -168,11 +224,14 @@ struct ConvGeom;
 bool autocorr_kernel_enabled();
 int debug_read_ac_counters(unsigned long long* out, int n);
 size_t autocorr_table_bytes(const ConvGeom* geoms, int n);
+// deterministic mode: autocorr_count adds the output tiles of the layers to det before the
+// build, which then gives every item whose tiles have other contributors its slots
+void autocorr_count(const ConvGeom* geoms, float* const* accs, int n, DetCombine* det);
 int autocorr_table_build(const ConvGeom* geoms, const float* const* stages, float* const* accs,
                          int n, void* table_dev, size_t table_bytes, SubGroup* sg,
-                         cudaStream_t stream);
+                         cudaStream_t stream, DetCombine* det = nullptr);
 int autocorr_launch(const void* table_dev, const SubGroup& sg, cudaStream_t stream,
-                    int max_ctas = 0, int pdl = 0);
+                    int max_ctas = 0, int pdl = 0, float* slots = nullptr);
 
 // engines
 int contraction_simt(const ContractionArgs& a, cudaStream_t stream);

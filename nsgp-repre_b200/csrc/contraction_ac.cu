@@ -53,11 +53,11 @@ struct alignas(64) AcProblem {
 };
 struct alignas(16) AcItem {
   int prob, pass, rb, cb;
-  int x0, u0, u1, pad;
+  int x0, u0, u1, slot;       // slot > 0: the tiles dy0..2 go to slots slot-1, slot, ...
 };
 
 // pass -> (A copy, B copy, dx, first dy)
-__device__ __forceinline__ void pass_info(int pass, int rb, int cb, int* sa, int* sb, int* dx,
+__host__ __device__ __forceinline__ void pass_info(int pass, int rb, int cb, int* sa, int* sb, int* dx,
                                           int* dy0) {
   *sa = pass == 3 ? 1 : (pass == 4 ? 2 : 0);
   *sb = pass == 1 ? 1 : (pass == 2 ? 2 : 0);
@@ -82,7 +82,8 @@ __device__ unsigned long long g_ac_counters[160 * 8];
 
 __global__ void __launch_bounds__(kThreadsAc, 1)
 autocorr_tc_kernel(const AcProblem* __restrict__ probs, const AcItem* __restrict__ items,
-                   int n_items, int dbg, unsigned long long* tl, int* __restrict__ sched) {
+                   int n_items, int dbg, unsigned long long* tl, int* __restrict__ sched,
+                   float* __restrict__ slots) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>(
       (reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -305,6 +306,10 @@ autocorr_tc_kernel(const AcProblem* __restrict__ probs, const AcItem* __restrict
       for (int dy = dy0; dy < 3; ++dy) {
         float* mat = p.acc + (long long)ac_ridx(dy, dx) * C * p.ldc;
         float* orow = mat + (long long)row * p.ldc;
+        // deterministic mode: the partial tile goes to its slot (zeros where masked)
+        float* srow = it.slot > 0 ? slots + (size_t)(it.slot - 1 + dy - dy0) * kSlotElems +
+                                        (quad * 32 + lane) * 128
+                                  : nullptr;
 #pragma unroll 1
         for (int chunk = 0; chunk < BM / 32; ++chunk) {
           uint32_t v[32];
@@ -312,7 +317,18 @@ autocorr_tc_kernel(const AcProblem* __restrict__ probs, const AcItem* __restrict
           tc_ld32(taddr, v);
           tc_wait_ld();
           const int col0 = it.cb * BM + chunk * 32;
-          if (row_ok && col0 < C) {
+          if (srow != nullptr) {
+#pragma unroll
+            for (int j = 0; j < 32; j += 4) {
+              const int col = col0 + j;
+              float4 x;
+              x.x = row_ok && col < C ? __uint_as_float(v[j]) : 0.f;
+              x.y = row_ok && col + 1 < C ? __uint_as_float(v[j + 1]) : 0.f;
+              x.z = row_ok && col + 2 < C ? __uint_as_float(v[j + 2]) : 0.f;
+              x.w = row_ok && col + 3 < C ? __uint_as_float(v[j + 3]) : 0.f;
+              *reinterpret_cast<float4*>(srow + chunk * 32 + j) = x;
+            }
+          } else if (row_ok && col0 < C) {
 #pragma unroll
             for (int j = 0; j < 32; j += 4) {
               const int col = col0 + j;
@@ -391,13 +407,39 @@ size_t autocorr_table_bytes(const ConvGeom* geoms, int n) {
     const size_t t = (size_t)ceil_div(g.C, BM);
     items += 5 * t * t * (size_t)ceil_div(g.W, BK) * (size_t)ceil_div(g.H, kRowsPerItem);
   }
-  return (size_t)n * sizeof(AcProblem) + items * sizeof(AcItem) + 1024;
+  // deterministic mode: up to three partial tiles per item
+  return (size_t)n * sizeof(AcProblem) + items * sizeof(AcItem) + 1024 +
+         (g_deterministic ? DetCombine::bytes_bound(3 * items) : 0);
+}
+
+// output tile of (layer accumulator, pass, dy, tile) - the address the epilogue adds into
+static float* ac_tile(float* acc, const ConvGeom& g, int pass, int dy, int rb, int cb) {
+  int sa, sb, dx, dy0;
+  pass_info(pass, rb, cb, &sa, &sb, &dx, &dy0);
+  const int ldc = (int)round_up(g.C, 4);
+  return acc + (long long)ac_ridx(dy, dx) * g.C * ldc + (long long)rb * BM * ldc + cb * BM;
+}
+
+void autocorr_count(const ConvGeom* geoms, float* const* accs, int n, DetCombine* det) {
+  for (int i = 0; i < n; ++i) {
+    const ConvGeom& g = geoms[i];
+    const int tiles = ac_cblocks(g), strips = ceil_div(g.W, BK);
+    for (int u0 = 0; u0 < g.H; u0 += kRowsPerItem)
+      for (int st = 0; st < strips; ++st)
+        for (int pass = 0; pass < 5; ++pass)
+          for (int rb = 0; rb < tiles; ++rb)
+            for (int cb = 0; cb < tiles; ++cb) {
+              int sa, sb, dx, dy0;
+              pass_info(pass, rb, cb, &sa, &sb, &dx, &dy0);
+              for (int dy = dy0; dy < 3; ++dy) det->count(ac_tile(accs[i], g, pass, dy, rb, cb));
+            }
+  }
 }
 
 // geoms[i] / stages[i] / accs[i]: staged autocorrelation layers.  Uploads the table.
 int autocorr_table_build(const ConvGeom* geoms, const float* const* stages, float* const* accs,
                          int n, void* table_dev, size_t table_bytes, SubGroup* sg,
-                         cudaStream_t stream) {
+                         cudaStream_t stream, DetCombine* det) {
   EncodeTiledFn enc = encode_fn();
   NSGP_REQUIRE(enc != nullptr, "autocorr kernel: cuTensorMapEncodeTiled is unavailable");
   std::vector<AcProblem> hp(n);
@@ -438,7 +480,24 @@ int autocorr_table_build(const ConvGeom* geoms, const float* const* stages, floa
               Key k;
               k.rows = u1 - u0; k.layer = i; k.u0 = u0; k.x0 = st * BK; k.pass = pass;
               k.tile = rb * p.tiles + cb;
-              k.it = AcItem{i, pass, rb, cb, st * BK, u0, u1, 0};
+              int slot = 0;
+              if (det != nullptr) {
+                int sa, sb, dx, dy0;
+                pass_info(pass, rb, cb, &sa, &sb, &dx, &dy0);
+                bool shared = false;
+                for (int dy = dy0; dy < 3; ++dy)
+                  shared |= det->contributors(ac_tile(accs[i], g, pass, dy, rb, cb)) > 1;
+                if (shared) {
+                  // consecutive slots, one per tile dy0..2
+                  const int rows = g.C - rb * BM, cols = g.C - cb * BM;
+                  for (int dy = dy0; dy < 3; ++dy) {
+                    const int s = det->assign(ac_tile(accs[i], g, pass, dy, rb, cb), p.ldc,
+                                              rows < BM ? rows : BM, cols < BM ? cols : BM);
+                    if (dy == dy0) slot = s + 1;
+                  }
+                }
+              }
+              k.it = AcItem{i, pass, rb, cb, st * BK, u0, u1, slot};
               keys.push_back(k);
             }
     }
@@ -475,7 +534,7 @@ int autocorr_table_build(const ConvGeom* geoms, const float* const* stages, floa
 }
 
 int autocorr_launch(const void* table_dev, const SubGroup& sg, cudaStream_t stream, int max_ctas,
-                    int pdl) {
+                    int pdl, float* slots) {
   if (sg.n_items == 0) return 0;
   static bool configured = false;
   if (!configured) {
@@ -503,7 +562,7 @@ int autocorr_launch(const void* table_dev, const SubGroup& sg, cudaStream_t stre
   int* sched = reinterpret_cast<int*>(const_cast<char*>((const char*)table_dev) + sg.off_items +
                                       (size_t)sg.n_items * sizeof(AcItem));
   NSGP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, autocorr_tc_kernel, probs, items, sg.n_items, dbg,
-                                     timeline_slot(10), sched));
+                                     timeline_slot(10), sched, slots));
   NSGP_LAUNCHED();
   return 0;
 }

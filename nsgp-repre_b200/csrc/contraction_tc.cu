@@ -60,6 +60,7 @@ struct Item {
   const TcMaps* maps;
   const TcParams* p;
   int rb, cb, kb0, kb1;
+  int slot;                  // > 0: partial tile goes to slot (slot - 1), see DetCombine
 };
 
 // Single problem: items are (K split, tile) pairs enumerated arithmetically; Gram
@@ -70,14 +71,16 @@ __device__ __forceinline__ Item fetch_item(const TcMaps* pmaps, const TcParams* 
   Item it;
   if (gitems != nullptr) {
     const int4 a = *reinterpret_cast<const int4*>(&gitems[idx]);
-    const int kb1 = gitems[idx].kb1;
+    const int4 b = *reinterpret_cast<const int4*>(&gitems[idx].kb1);
     it.maps = &gprobs[a.x].maps;
     it.p = &gprobs[a.x].p;
-    it.rb = a.y; it.cb = a.z; it.kb0 = a.w; it.kb1 = kb1;
+    it.rb = a.y; it.cb = a.z; it.kb0 = a.w; it.kb1 = b.x;
+    it.slot = b.y;
     return it;
   }
   it.maps = pmaps;
   it.p = pp;
+  it.slot = 0;
   const int split = idx / pp->n_tiles;
   int tile = idx - split * pp->n_tiles;
   if (pp->gram) {
@@ -116,7 +119,8 @@ __global__ void __launch_bounds__(kThreads, 1)
 contraction_tc_kernel(const __grid_constant__ TcMaps pmaps, const __grid_constant__ TcParams pp,
                       const TcProblem* __restrict__ gprobs, const TcItem* __restrict__ gitems,
                       int n_items_max, int dbg,
-                      unsigned long long* tl, const int* __restrict__ n_items_dev) {
+                      unsigned long long* tl, const int* __restrict__ n_items_dev,
+                      float* __restrict__ slots) {
   // the item count may live in device memory (work lists generated on the device)
   const int n_items = n_items_dev != nullptr ? min(n_items_max, __ldg(n_items_dev)) : n_items_max;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -352,6 +356,10 @@ contraction_tc_kernel(const __grid_constant__ TcMaps pmaps, const __grid_constan
       const int n_cols = p.n_cols;
       const bool vec = p.vec_red != 0;
       const bool gram = p.gram != 0;
+      // deterministic mode: the whole partial tile goes to its slot (zeros where masked)
+      float* srow = (!PAIR && it.slot > 0)
+                        ? slots + (size_t)(it.slot - 1) * kSlotElems + (quad * 32 + lane) * 128
+                        : nullptr;
 #pragma unroll 1
       for (int chunk = 0; chunk < TILE / 32; ++chunk) {
         uint32_t v[32];
@@ -370,7 +378,19 @@ contraction_tc_kernel(const __grid_constant__ TcMaps pmaps, const __grid_constan
         const int col0 = it.cb * TILE + chunk * 32;
         // Gram: chunks strictly left of this CTA's diagonal block carry nothing needed
         const bool wanted = !gram || (col0 + 31 >= rblk);
-        if (row_ok && col0 < n_cols && wanted) {
+        if (srow != nullptr) {
+          const bool ok = row_ok && wanted;
+#pragma unroll
+          for (int j = 0; j < 32; j += 4) {
+            const int col = col0 + j;
+            float4 x;
+            x.x = ok && col < n_cols ? alpha * __uint_as_float(v[j]) : 0.f;
+            x.y = ok && col + 1 < n_cols ? alpha * __uint_as_float(v[j + 1]) : 0.f;
+            x.z = ok && col + 2 < n_cols ? alpha * __uint_as_float(v[j + 2]) : 0.f;
+            x.w = ok && col + 3 < n_cols ? alpha * __uint_as_float(v[j + 3]) : 0.f;
+            *reinterpret_cast<float4*>(srow + chunk * 32 + j) = x;
+          }
+        } else if (row_ok && col0 < n_cols && wanted) {
 #pragma unroll
           for (int j = 0; j < 32; j += 4) {
             const int col = col0 + j;
@@ -505,7 +525,8 @@ int configure_kernel() {
 // Launch over `n_items` work items with `workers` CTAs (single) or CTA pairs (pair).
 int launch_kernel(bool pair, const TcMaps& maps, const TcParams& p, const TcProblem* gprobs,
                   const TcItem* gitems, int n_items, int kind, cudaStream_t stream,
-                  int max_ctas = 0, int pdl = 0, const int* n_items_dev = nullptr) {
+                  int max_ctas = 0, int pdl = 0, const int* n_items_dev = nullptr,
+                  float* slots = nullptr) {
   if (n_items <= 0) return 0;
   ProfScope prof(kind, stream);
 #ifndef NSGP_BRINGUP
@@ -530,7 +551,8 @@ int launch_kernel(bool pair, const TcMaps& maps, const TcParams& p, const TcProb
     cfg.numAttrs = 1;
     NSGP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, contraction_tc_kernel<true>, maps, p, gprobs, gitems,
                                        n_items, dbg_counters(),
-                                       (unsigned long long*)nullptr, (const int*)nullptr));
+                                       (unsigned long long*)nullptr, (const int*)nullptr,
+                                       (float*)nullptr));
     NSGP_LAUNCHED();
     return 0;
   }
@@ -553,7 +575,7 @@ int launch_kernel(bool pair, const TcMaps& maps, const TcParams& p, const TcProb
     NSGP_CHECK_CUDA(cudaLaunchKernelEx(&cfg, contraction_tc_kernel<false>, maps, p, gprobs, gitems,
                                        n_items, dbg_counters(),
                                        kind == kProfGram ? timeline_slot(0) : nullptr,
-                                       n_items_dev));
+                                       n_items_dev, slots));
   }
   NSGP_LAUNCHED();
   return 0;
@@ -579,7 +601,7 @@ bool want_pair(const ContractionArgs& a) {
   const bool gram = a.epi == kEpiGramAtomic;
   const bool same = gram && a.A.base == a.B.base && a.A.hl_stride == a.B.hl_stride &&
                     a.A.rows == a.B.rows;
-  if (force == 0) return false;
+  if (force == 0 || g_deterministic) return false;   // the pair kernel has no slot epilogue
   if (force == 3) return a.A.rows > 128;
   if (force == 1) return gram && same;
   // default: autocorrelation-layout problems (they carry an l2_group) on 256-multiples
@@ -695,6 +717,13 @@ int contraction_tc(const ContractionArgs& a, cudaStream_t stream) {
       if (best < 0 || cost < best) { best = cost; best_s = sp; }
     }
     p.splits = best_s;
+    // deterministic mode: one item per output tile, whose red.add is then the only addend
+    if (g_deterministic) {
+      NSGP_REQUIRE(s_min == 1, "deterministic mode: a single-problem contraction over %d K "
+                   "blocks needs a K split; it has no deterministic form (use a group table)",
+                   p.nkb);
+      p.splits = 1;
+    }
   }
   return launch_kernel(pair, prob.maps, p, nullptr, nullptr, p.n_tiles * p.splits,
                        p.gram ? kProfGram : kProfGemm, stream);
@@ -709,7 +738,7 @@ int debug_read_counters(unsigned long long* out, int n) {
 // A group table holds up to two sub-tables: problems run by the single-CTA kernel and
 // problems run by the CTA-pair kernel (one launch each).
 size_t group_table_bytes(const ContractionArgs* probs, int n) {
-  size_t items = 0;
+  size_t items = 0, det_items = 0;
   for (int i = 0; i < n; ++i) {
     const int tm = ceil_div(probs[i].A.rows, BM), tn = ceil_div(probs[i].n_cols, BN);
     const int nkb = k_blocks(probs[i].A);
@@ -719,15 +748,45 @@ size_t group_table_bytes(const ContractionArgs* probs, int n) {
     const int chain = probs[i].chain > 0 ? (probs[i].chain < 32 ? probs[i].chain : 32)
                                          : (gram ? 32 : kChainGemm);
     items += tiles * (size_t)ceil_div(nkb > 0 ? nkb : 1, chain);
+    // deterministic mode (single-CTA kernel only): exact item count, each may need a slot
+    const int chain_d = probs[i].chain > 0 ? probs[i].chain : (gram ? kChainGram : kChainGemm);
+    det_items += tiles * (size_t)ceil_div(nkb > 0 ? nkb : 1, chain_d);
   }
-  return (size_t)n * sizeof(TcProblem) + items * sizeof(TcItem) + 1024;
+  return (size_t)n * sizeof(TcProblem) + items * sizeof(TcItem) + 1024 +
+         (g_deterministic ? DetCombine::bytes_bound(det_items) : 0);
+}
+
+// Output tiles of every work item of the problems, as group_table_build enumerates them in
+// deterministic mode (single-CTA kernel)
+void group_table_count(const ContractionArgs* probs, int n, DetCombine* det) {
+  for (int i = 0; i < n; ++i) {
+    const ContractionArgs& a = probs[i];
+    const int nkb = k_blocks(a.A);
+    if (a.A.rows == 0 || a.n_cols == 0 || nkb == 0) continue;
+    const bool gram = a.epi == kEpiGramAtomic;
+    const int tm = ceil_div(a.A.rows, BM), tn = ceil_div(a.n_cols, BN);
+    const int chain = a.chain > 0 ? a.chain : (gram ? kChainGram : kChainGemm);
+    const int splits = ceil_div(nkb, chain);
+    for (int sp = 0; sp < splits; ++sp)
+      for (int rb = 0; rb < tm; ++rb)
+        for (int cb = gram ? rb : 0; cb < tn; ++cb)
+          det->count(a.out + (long long)rb * BM * a.ld + cb * BN);
+  }
 }
 
 int group_table_build(const ContractionArgs* probs, int n, int kind, void* table_dev,
-                      size_t table_bytes, GroupInfo* info, cudaStream_t stream) {
+                      size_t table_bytes, GroupInfo* info, cudaStream_t stream, DetCombine* det) {
   NSGP_REQUIRE((probs || n == 0) && table_dev && info && n >= 0, "group_build: bad arguments");
   NSGP_REQUIRE((reinterpret_cast<uintptr_t>(table_dev) & 63) == 0,
                "group_build: table must be 64-byte aligned");
+  // deterministic mode: the slots of this launch, counted here unless the caller shares the
+  // combine with another sub-table
+  DetCombine local;
+  const bool own_det = det == nullptr && g_deterministic;
+  if (own_det) {
+    det = &local;
+    group_table_count(probs, n, det);
+  }
   struct Cost { long long c; int grp, split; TcItem it; };
   std::vector<TcProblem> hp[2];
   std::vector<Cost> items[2];
@@ -747,7 +806,16 @@ int group_table_build(const ContractionArgs* probs, int n, int kind, void* table
       for (int rb = 0; rb < p.tiles_m; ++rb)
         for (int cb = p.gram ? rb : 0; cb < p.tiles_n; ++cb) {
           Cost c;
-          c.it = TcItem{prob, rb, cb, kb0, kb1, 0, 0, 0};
+          int slot = 0;
+          if (det != nullptr) {
+            NSGP_REQUIRE(k == 0, "group_build: deterministic tables use the single-CTA kernel");
+            float* tile = a.out + (long long)rb * BM * a.ld + cb * BN;
+            if (det->contributors(tile) > 1) {
+              const int rows = a.A.rows - rb * BM, cols = a.n_cols - cb * BN;
+              slot = 1 + det->assign(tile, a.ld, rows < BM ? rows : BM, cols < BN ? cols : BN);
+            }
+          }
+          c.it = TcItem{prob, rb, cb, kb0, kb1, slot, 0, 0};
           c.c = (long long)(kb1 - kb0) * 8 + 16;       // ~ K blocks + a fixed part
           c.grp = a.l2_group > 0 ? a.l2_group : -(i + 1);
           c.split = sp;
@@ -775,9 +843,15 @@ int group_table_build(const ContractionArgs* probs, int n, int kind, void* table
     off = (size_t)round_up((long long)(sg.off_items + items[k].size() * sizeof(TcItem)), 64);
   }
   info->sub[2] = SubGroup{0, 0, 0, 0};
+  info->sub[3] = SubGroup{0, 0, 0, 0};
+  if (own_det) off = local.layout(off, &info->sub[3]);
   info->bytes = off;
   NSGP_REQUIRE(info->bytes <= table_bytes, "group_build: table too small (%zu < %zu)",
                table_bytes, info->bytes);
+  if (own_det) {
+    int rc = det_combine_upload(local, table_dev, info->sub[3], stream);
+    if (rc) return rc;
+  }
   for (int k = 0; k < 2; ++k) {
     const SubGroup& sg = info->sub[k];
     if (sg.n_items == 0) continue;
@@ -792,28 +866,35 @@ int group_table_build(const ContractionArgs* probs, int n, int kind, void* table
   return 0;
 }
 
+static float* group_slots(const void* table_dev, const GroupInfo& info) {
+  if (info.sub[3].n_items == 0) return nullptr;
+  return reinterpret_cast<float*>(const_cast<char*>((const char*)table_dev) + info.sub[3].off_probs);
+}
+
 int group_launch_sub(const void* table_dev, const GroupInfo& info, int which, int max_ctas,
                      int pdl, cudaStream_t stream) {
   static const TcMaps dummy_maps{};
   TcParams dummy{};
-  if (which == 2) return autocorr_launch(table_dev, info.sub[2], stream, max_ctas, pdl);
+  float* slots = group_slots(table_dev, info);
+  if (which == 2) return autocorr_launch(table_dev, info.sub[2], stream, max_ctas, pdl, slots);
   const SubGroup& sg = info.sub[0];
   if (sg.n_items == 0) return 0;
   const TcProblem* probs = reinterpret_cast<const TcProblem*>((const char*)table_dev + sg.off_probs);
   const TcItem* items = reinterpret_cast<const TcItem*>((const char*)table_dev + sg.off_items);
   return launch_kernel(false, dummy_maps, dummy, probs, items, sg.n_items, info.kind, stream,
-                       max_ctas, pdl);
+                       max_ctas, pdl, nullptr, slots);
 }
 
 // one problem, work items written by a device kernel (at most max_items of them, the live
 // count in *n_items_dev): RePRE's Gram over the class-sorted foreground rows
 int contraction_launch_dev_items(const void* prob_dev, const void* items_dev, int max_items,
-                                 const int* n_items_dev, int kind, cudaStream_t stream) {
+                                 const int* n_items_dev, int kind, float* slots,
+                                 cudaStream_t stream) {
   static const TcMaps dummy_maps{};
   TcParams dummy{};
   return launch_kernel(false, dummy_maps, dummy, reinterpret_cast<const TcProblem*>(prob_dev),
                        reinterpret_cast<const TcItem*>(items_dev), max_items, kind, stream, 0, 0,
-                       n_items_dev);
+                       n_items_dev, slots);
 }
 // host part of the same: validates the problem and encodes its tensor maps
 int contraction_build_problem(const ContractionArgs& a, void* prob_host /* TcProblem */) {
@@ -827,17 +908,103 @@ size_t contraction_item_bytes() { return sizeof(TcItem); }
 int group_launch(const void* table_dev, const GroupInfo& info, cudaStream_t stream) {
   static const TcMaps dummy_maps{};
   TcParams dummy{};
+  float* slots = group_slots(table_dev, info);
   for (int k = 1; k >= 0; --k) {          // pair sub-table first: it holds the big layers
     const SubGroup& sg = info.sub[k];
     if (sg.n_items == 0) continue;
     const TcProblem* probs = reinterpret_cast<const TcProblem*>((const char*)table_dev + sg.off_probs);
     const TcItem* items = reinterpret_cast<const TcItem*>((const char*)table_dev + sg.off_items);
-    int rc = launch_kernel(k == 1, dummy_maps, dummy, probs, items, sg.n_items, info.kind, stream);
+    int rc = launch_kernel(k == 1, dummy_maps, dummy, probs, items, sg.n_items, info.kind, stream,
+                           0, 0, nullptr, slots);
     if (rc) return rc;
   }
   // autocorrelation sub-table last: its long items fill the machine best once the small
   // problems are out of the way
-  return autocorr_launch(table_dev, info.sub[2], stream);
+  int rc = autocorr_launch(table_dev, info.sub[2], stream, 0, 0, slots);
+  if (rc) return rc;
+  return det_combine_launch(table_dev, info.sub[3], info.kind, stream);
+}
+
+// ---------------------------------------------------------------- ordered combine
+int DetCombine::assign(float* tile, int ld, int rows, int cols) {
+  auto it = tile_of.find(tile);
+  int t;
+  if (it == tile_of.end()) {
+    t = (int)tiles.size();
+    tile_of.emplace(tile, t);
+    CombTile c{};
+    c.out = tile; c.ld = ld; c.rows = rows; c.cols = cols;
+    tiles.push_back(c);
+    per_tile.emplace_back();
+  } else {
+    t = it->second;
+  }
+  per_tile[t].push_back(n_slots);
+  return n_slots++;
+}
+
+size_t DetCombine::layout(size_t off, SubGroup* sg) const {
+  off = (size_t)round_up((long long)off, 256);
+  sg->n_items = (int)tiles.size();
+  sg->off_items = off;
+  sg->n_problems = n_slots;
+  off += tiles.size() * sizeof(CombTile) + (size_t)n_slots * sizeof(int);
+  sg->off_probs = (size_t)round_up((long long)off, 256);
+  return sg->off_probs + (size_t)n_slots * kSlotElems * sizeof(float);
+}
+
+int det_combine_upload(const DetCombine& det, void* table_dev, const SubGroup& sg,
+                       cudaStream_t stream) {
+  if (sg.n_items == 0) return 0;
+  std::vector<CombTile> t(det.tiles);
+  std::vector<int> list;
+  list.reserve(det.n_slots);
+  for (size_t i = 0; i < t.size(); ++i) {
+    t[i].first = (int)list.size();
+    t[i].n = (int)det.per_tile[i].size();
+    list.insert(list.end(), det.per_tile[i].begin(), det.per_tile[i].end());
+  }
+  char* base = (char*)table_dev + sg.off_items;
+  NSGP_CHECK_CUDA(cudaMemcpyAsync(base, t.data(), t.size() * sizeof(CombTile),
+                                  cudaMemcpyHostToDevice, stream));
+  NSGP_CHECK_CUDA(cudaMemcpyAsync(base + t.size() * sizeof(CombTile), list.data(),
+                                  list.size() * sizeof(int), cudaMemcpyHostToDevice, stream));
+  return 0;
+}
+
+namespace {
+// One CTA per output tile: sum the tile's slots in list order, then one read-modify-write of
+// the running sum.  The contraction launch before it on the stream wrote the slots.
+__global__ void __launch_bounds__(256)
+det_combine_kernel(const CombTile* __restrict__ tiles, const float* __restrict__ slots) {
+  const CombTile t = tiles[blockIdx.x];
+  const int* ids = reinterpret_cast<const int*>(tiles + gridDim.x) + t.first;
+  for (int e = threadIdx.x; e < kSlotElems / 4; e += 256) {
+    const int r = e >> 5, c = (e & 31) * 4;
+    if (r >= t.rows || c >= t.cols) continue;
+    const size_t off = (size_t)r * 128 + c;
+    float4 s = *reinterpret_cast<const float4*>(slots + (size_t)ids[0] * kSlotElems + off);
+    for (int k = 1; k < t.n; ++k) {
+      const float4 v = *reinterpret_cast<const float4*>(slots + (size_t)ids[k] * kSlotElems + off);
+      s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
+    }
+    float* o = t.out + (long long)r * t.ld + c;
+    o[0] += s.x;
+    if (c + 1 < t.cols) o[1] += s.y;
+    if (c + 2 < t.cols) o[2] += s.z;
+    if (c + 3 < t.cols) o[3] += s.w;
+  }
+}
+}  // namespace
+
+int det_combine_launch(const void* table_dev, const SubGroup& sg, int kind, cudaStream_t stream) {
+  if (sg.n_items == 0) return 0;
+  ProfScope prof(kind, stream);
+  det_combine_kernel<<<sg.n_items, 256, 0, stream>>>(
+      reinterpret_cast<const CombTile*>((const char*)table_dev + sg.off_items),
+      reinterpret_cast<const float*>((const char*)table_dev + sg.off_probs));
+  NSGP_LAUNCHED();
+  return 0;
 }
 
 }  // namespace nsgp

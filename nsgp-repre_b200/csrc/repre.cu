@@ -143,8 +143,9 @@ int launch_segment_mean(const float* F, int D, const int* seg_off, const int* ro
   if (nseg == 0) return 0;
   int chunks = ceil_div(D, kSegThreads * 4);
   int splits = 1;
-  // fill the 148 SMs a few times over when there are few / long segments
-  while (splits < 32 && (long long)chunks * nseg * splits < 148 * 8 &&
+  // fill the 148 SMs a few times over when there are few / long segments (row-split partial
+  // means meet by atomicAdd, so deterministic mode keeps one sequential pass per segment)
+  while (!g_deterministic && splits < 32 && (long long)chunks * nseg * splits < 148 * 8 &&
          max_seg_rows / (splits * 2) >= 16)
     splits *= 2;
   if (splits > 1)
@@ -560,7 +561,7 @@ repre_plan_kernel(const int* __restrict__ offsets, int class_first, int n_classe
                   const int* __restrict__ n_saved, const int* __restrict__ saved_len, int nkb,
                   int max_items, ClassExtent* __restrict__ ext, GreedyClass* __restrict__ cls,
                   int2* __restrict__ pairs, tc::TcItem* __restrict__ items,
-                  tc::TcProblem* __restrict__ prob, int* __restrict__ hdr) {
+                  tc::TcProblem* __restrict__ prob, int* __restrict__ hdr, int det) {
   __shared__ int s_npairs, s_splits;
   extern __shared__ int plan_smem[];          // [n_classes + 1] offsets, [n] n_saved, [n] saved_len
   int* s_o = plan_smem;
@@ -608,8 +609,10 @@ repre_plan_kernel(const int* __restrict__ offsets, int class_first, int n_classe
     // few tile pairs, so that every SM gets a couple of items
     int splits = (nkb + 63) / 64;
     const int want = np > 0 ? (2 * 148) / np : 1;      // at most two full waves of items
-    if (want > splits) splits = want;
-    if (splits > nkb / 4) splits = nkb / 4 > 0 ? nkb / 4 : 1;
+    // deterministic mode: only the splits the chain bound needs (their partial tiles go to
+    // slots and are summed in split order by repre_combine_tiles_kernel)
+    if (want > splits && !det) splits = want;
+    if (splits > nkb / 4 && !det) splits = nkb / 4 > 0 ? nkb / 4 : 1;
     while (np * splits > max_items && splits > 1) --splits;
     s_npairs = np;
     s_splits = splits;
@@ -625,7 +628,34 @@ repre_plan_kernel(const int* __restrict__ offsets, int class_first, int n_classe
     const int2 t = pairs[pr];                           // tiles is in flight together
     const int kb0 = (int)((long long)nkb * sp / splits);
     const int kb1 = (int)((long long)nkb * (sp + 1) / splits);
-    items[i] = tc::TcItem{0, t.x, t.y, kb0, kb1, 0, 0, 0};
+    items[i] = tc::TcItem{0, t.x, t.y, kb0, kb1, det && splits > 1 ? i + 1 : 0, 0, 0};
+  }
+}
+
+// deterministic mode: S tile of pair p += sum over the K splits of slots[sp * np + p], in split
+// order (the plan gave item i = sp * np + p slot i)
+__global__ void __launch_bounds__(256)
+repre_combine_tiles_kernel(const int2* __restrict__ pairs, const int* __restrict__ hdr,
+                           const float* __restrict__ slots, float* __restrict__ S, int ld_s) {
+  const int np = hdr[1], n_fg = hdr[0], splits = hdr[4];
+  if (splits <= 1) return;
+  for (int p = blockIdx.x; p < np; p += gridDim.x) {
+    const int2 t = pairs[p];
+    for (int e = threadIdx.x; e < 128 * 32; e += 256) {
+      const int r = t.x * 128 + (e >> 5), c = t.y * 128 + (e & 31) * 4;
+      if (r >= n_fg || c >= ld_s) continue;
+      const size_t off = (size_t)(e >> 5) * 128 + (e & 31) * 4;
+      float4 s = *reinterpret_cast<const float4*>(slots + (size_t)p * kSlotElems + off);
+      for (int sp = 1; sp < splits; ++sp) {
+        const float4 v =
+            *reinterpret_cast<const float4*>(slots + ((size_t)sp * np + p) * kSlotElems + off);
+        s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
+      }
+      float4* o = reinterpret_cast<float4*>(S + (long long)r * ld_s + c);
+      float4 a = *o;
+      a.x += s.x; a.y += s.y; a.z += s.z; a.w += s.w;
+      *o = a;
+    }
   }
 }
 
@@ -718,13 +748,13 @@ threshold_count_dev_kernel(const float* __restrict__ S_all, const ClassExtent* _
 int launch_repre_plan(const int* offsets, int class_first, int n_classes, int ld_s,
                       const int* n_saved_dev, const int* saved_len_dev, int nkb, int max_items,
                       ClassExtent* ext, GreedyClass* cls, void* pairs, void* items, void* prob,
-                      int* hdr, cudaStream_t stream) {
+                      int* hdr, int det, cudaStream_t stream) {
   ProfScope prof(kProfRepre, stream);
   repre_plan_kernel<<<1, 256, (3 * n_classes + 1) * sizeof(int), stream>>>(offsets, class_first, n_classes, ld_s, n_saved_dev,
                                            saved_len_dev, nkb, max_items, ext, cls,
                                            reinterpret_cast<int2*>(pairs),
                                            reinterpret_cast<tc::TcItem*>(items),
-                                           reinterpret_cast<tc::TcProblem*>(prob), hdr);
+                                           reinterpret_cast<tc::TcProblem*>(prob), hdr, det);
   NSGP_LAUNCHED();
   return 0;
 }
@@ -737,6 +767,15 @@ int launch_repre_prepare(const float* F, int D, int M, const int* rows, const in
                                                         S, ld_s);
   NSGP_LAUNCHED();
   normalize_split_dev_kernel<<<M, 256, 0, stream>>>(F, D, rows, offsets, class_first, hdr, hi, lo);
+  NSGP_LAUNCHED();
+  return 0;
+}
+
+int launch_repre_combine(const void* pairs, const int* hdr, const float* slots, float* S, int ld_s,
+                         cudaStream_t stream) {
+  ProfScope prof(kProfRepre, stream);
+  repre_combine_tiles_kernel<<<148 * 2, 256, 0, stream>>>(reinterpret_cast<const int2*>(pairs),
+                                                          hdr, slots, S, ld_s);
   NSGP_LAUNCHED();
   return 0;
 }

@@ -42,7 +42,10 @@ int launch_class_index_fused(const long long* labels, int M, int C, int* counts,
 int launch_repre_plan(const int* offsets, int class_first, int n_classes, int ld_s,
                       const int* n_saved_dev, const int* saved_len_dev, int nkb, int max_items,
                       ClassExtent* ext, GreedyClass* cls, void* pairs, void* items, void* prob,
-                      int* hdr, cudaStream_t s);
+                      int* hdr, int det, cudaStream_t s);
+// deterministic mode: the K-split partial Gram tiles (slots) summed into S in split order
+int launch_repre_combine(const void* pairs, const int* hdr, const float* slots, float* S, int ld_s,
+                         cudaStream_t s);
 int launch_repre_prepare(const float* F, int D, int M, const int* rows, const int* offsets,
                          int class_first, const int* hdr, float* hi, float* lo,
                          const void* pairs, float* S, int ld_s, cudaStream_t s);

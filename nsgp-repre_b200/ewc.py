@@ -40,11 +40,13 @@ def register_params(model, must_names=("bn",), ignore_names=("teacher_model",)) 
 
 
 def _table(n: int, device, cache: dict) -> torch.Tensor:
+    # deterministic mode: the table also holds the penalty's fp64 partial sums
+    det = _lib.deterministic()
     need = int(lib.nsgp_ewc_table_bytes(n))
     t = cache.get("table")
-    if t is None or t.numel() < need or t.device != device:
+    if t is None or t.numel() < need or t.device != device or cache.get("det") != det:
         t = torch.empty(need, dtype=torch.uint8, device=device)
-        cache["table"] = t
+        cache["table"], cache["det"] = t, det
     return t
 
 

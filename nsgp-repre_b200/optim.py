@@ -203,10 +203,11 @@ class SGDNSCL(Optimizer):
             self._stage[name] = st
         return st
 
-    def _build_group_cache(self, gi, group, device):
+    def _build_group_cache(self, gi, group, device, det):
         """Everything of a param group that survives from step to step: the ctypes tensor /
         layer tables, the T arena of its low-rank layers and the prepared plan.  Rebuilt when a
-        parameter, a projector or the set of names changes (``_group_key``)."""
+        parameter, a projector, the set of names or the deterministic mode (``det``, the plan's
+        K-split partial tiles meet in a fixed order) changes."""
         names, params = group["names"], group["params"]
         n_t = len(params)
         tensors = (SgdTensor * n_t)()
@@ -254,7 +255,7 @@ class SGDNSCL(Optimizer):
                      t_elems=t_elems, protos=protos, w_ptrs=[p.data_ptr() for p in params],
                      g_ptrs=[0] * n_t, buf_ptrs=[0] * n_t, first=[-1] * n_t, plan=None,
                      buf=None, names=list(names), n_transforms=len(self.transforms),
-                     uploaded=False)
+                     uploaded=False, det=det)
         if _lib.engine() == 0:
             # ctypes fields read 0 until the first step fills g / buf; the plan only encodes the
             # weights, projectors and staging buffers
@@ -271,9 +272,9 @@ class SGDNSCL(Optimizer):
         self._plans[gi] = cache
         return cache
 
-    def _group_cache_valid(self, cache, group) -> bool:
+    def _group_cache_valid(self, cache, group, det) -> bool:
         if cache is None or cache["names"] != group["names"] or \
-                cache["n_transforms"] != len(self.transforms):
+                cache["n_transforms"] != len(self.transforms) or cache["det"] != det:
             return False
         for p, w in zip(group["params"], cache["w_ptrs"]):
             if p.data_ptr() != w:
@@ -319,9 +320,10 @@ class SGDNSCL(Optimizer):
                         raise RuntimeError("mat1 and mat2 shapes cannot be multiplied "
                                            "(%dx%d and %dx%d)" % (cout, dd, P.shape[0], P.shape[1]))
                 grads.append(grad)
+            det = _lib.deterministic()
             cache = self._plans.get(gi)
-            if not self._group_cache_valid(cache, group):
-                cache = self._build_group_cache(gi, group, device)
+            if not self._group_cache_valid(cache, group, det):
+                cache = self._build_group_cache(gi, group, device, det)
             tensors = cache["tensors"]
             changed = not cache["uploaded"]
             g_ptrs, buf_ptrs, first = cache["g_ptrs"], cache["buf_ptrs"], cache["first"]

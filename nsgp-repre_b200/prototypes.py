@@ -119,8 +119,12 @@ class MultiPrototypeReplay:
         c0 = previous_cls[0]
         C = previous_cls[-1] + 1
         mp = self.max_proto - 1
+        # deterministic mode: the Gram's K-split partial tiles meet in split order and the
+        # segment means are one sequential pass per segment; the workspace (and a recorded
+        # graph) belongs to one mode
+        det = _lib.deterministic()
         need = int(lib.repre_build_prototypes_workspace_bytes(M, D, ncls, mp))
-        key = (M, D, C, ncls, mp, dev)
+        key = (M, D, C, ncls, mp, dev, det)
         if self._bufs is None or self._bufs[0] != key:
             nseg_max = ncls * (mp + 1)
             self._bufs = (key, dict(
@@ -239,6 +243,7 @@ class MultiPrototypeReplay:
         off_t, all_rows, max_rows = self._segments
         nseg, D = self.bbox_featss.shape
         var = torch.empty_like(self.bbox_featss)
+        _lib.deterministic()
         check(lib.repre_segment_var(ptr(self._feats), D, ptr(off_t), ptr(all_rows), nseg,
                                     int(max_rows), ptr(self.bbox_featss), ptr(var),
                                     _lib.current_stream(var.device)), "repre_segment_var")
@@ -360,6 +365,8 @@ def kmeans_prototypes(feats: torch.Tensor, init_centres: torch.Tensor, iters: in
     lowest k) through the tcgen05 contraction X C^T, update = segmented mean of the rows of
     every cluster (an empty cluster keeps its centre).  Returns (centres (k,D), labels (n,))."""
     _lib.require_cuda(feats, "features")
+    _lib.alert_not_deterministic("kmeans_prototypes")
+    _lib.deterministic()
     dev = feats.device
     x = feats.detach().reshape(feats.shape[0], -1)
     if x.dtype != torch.float32 or not x.is_contiguous():

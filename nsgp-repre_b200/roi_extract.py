@@ -44,6 +44,8 @@ class _RoIAlignFn(torch.autograd.Function):
         ext = ctx.ext
         (rois,) = ctx.saved_tensors
         dev = grad_out.device
+        # the transpose scatters with atomicAdd (as torchvision's roi_align backward does)
+        _lib.alert_not_deterministic("repre_roi_align_backward")
         L = len(ctx.shapes)
         grads = [torch.zeros(sh, dtype=torch.float32, device=dev) for sh in ctx.shapes]
         R = rois.shape[0]
@@ -176,7 +178,9 @@ class SingleRoIExtractor(nn.Module):
     def class_sums(self, feats, rois, labels, num_classes, return_feats=False):
         """RoIAlign fused with the per-class sums: returns (sums (num_classes, C*7*7),
         counts (num_classes,) int32[, feats (R, C*7*7)]); ``sums / counts`` are the coarse
-        prototypes ``mean(F[label == c], 0)`` of standard_roi_replay_head.py:411-415."""
+        prototypes ``mean(F[label == c], 0)`` of standard_roi_replay_head.py:411-415.  The sums
+        are atomicAdd'ed: raises (warns) under ``torch.use_deterministic_algorithms(True)``."""
+        _lib.alert_not_deterministic("SingleRoIExtractor.class_sums")
         out, sums, counts, _ = self._launch(feats, rois, None, labels, num_classes, return_feats)
         return (sums, counts, out) if return_feats else (sums, counts)
 
