@@ -136,6 +136,16 @@ segment_mean_kernel(const float* __restrict__ F, int D, const int* __restrict__ 
   }
 }
 
+// zero the rows the row-split means add into: the live ones only when the segment count is
+// read on the device, so that the rows past it keep whatever the caller left there
+__global__ void __launch_bounds__(256)
+zero_live_rows_kernel(float* __restrict__ out, int D, int nseg, const int* __restrict__ nseg_dev) {
+  const long long n4 = (long long)min(*nseg_dev, nseg) * (D / 4);
+  float4* o = reinterpret_cast<float4*>(out);
+  for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < n4; i += (long long)gridDim.x * 256)
+    o[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+}
+
 int launch_segment_mean(const float* F, int D, const int* seg_off, const int* rows, int nseg,
                         int max_seg_rows, const float* mu, int mode, float* out,
                         cudaStream_t stream, const int* nseg_dev) {
@@ -148,8 +158,13 @@ int launch_segment_mean(const float* F, int D, const int* seg_off, const int* ro
   while (!g_deterministic && splits < 32 && (long long)chunks * nseg * splits < 148 * 8 &&
          max_seg_rows / (splits * 2) >= 16)
     splits *= 2;
-  if (splits > 1)
+  if (splits > 1 && nseg_dev == nullptr) {
     NSGP_CHECK_CUDA(cudaMemsetAsync(out, 0, (size_t)nseg * D * sizeof(float), stream));
+  } else if (splits > 1) {
+    const int blocks = (int)std::min<long long>(ceil_div((long long)nseg * (D / 4), 256), 148 * 4);
+    zero_live_rows_kernel<<<blocks, 256, 0, stream>>>(out, D, nseg, nseg_dev);
+    NSGP_LAUNCHED();
+  }
   dim3 grid(chunks, nseg, splits);
   ProfScope prof(kProfRepre, stream);
   if (mode == 1)

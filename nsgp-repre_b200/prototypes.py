@@ -95,13 +95,10 @@ class MultiPrototypeReplay:
                 feats, labels, p, saved_masks) for p in parts]
             self.bbox_featss = torch.cat([m.bbox_featss for m in subs])
             self.tmp_label = torch.cat([m.tmp_label for m in subs])
+            # the runs in order walk previous_cls in order, as the reference's loop does
             merged = list(save_idx)
             for m in subs:
-                for c, masks in enumerate(m.save_idx):
-                    if c >= len(merged):
-                        merged.append(masks)
-                    elif masks and not merged[c]:
-                        merged[c] = masks
+                _place_masks(merged, m._class_masks())
             self.save_idx = merged
             self._segments, self._feats = None, feats
             return self
@@ -211,25 +208,28 @@ class MultiPrototypeReplay:
         """``mask.pth`` payload (:450-452): list[class] of list of bool masks over the
         class's rows; built from the device picks on first access."""
         if self._save_idx is None and self._lazy_masks is not None:
-            masks, counts, classes, npicks, picks, saved_lists, save_idx, mp = self._lazy_masks
-            h_cnt = counts.cpu().tolist()
-            sizes = [h_cnt[c] for c in classes]
-            moff = 0
-            for ci, (c, n) in enumerate(zip(classes, sizes)):
-                tmp = list(saved_lists[ci])
-                mine = [p for p in picks[ci * mp:ci * mp + npicks[ci]] if p >= 0]
-                if mine:
-                    idx = torch.tensor(mine, dtype=torch.int64, device=masks.device)
-                    sel = masks[moff:moff + n * n].view(n, n)[idx].cpu().bool()
-                    tmp.extend(sel[k].clone() for k in range(len(mine)))
-                moff += n * n
-                if c < len(save_idx):
-                    save_idx[c] = tmp
-                else:
-                    save_idx.append(tmp)
-            self._save_idx = save_idx
+            save_idx = self._lazy_masks[6]
+            self._save_idx = _place_masks(save_idx, self._class_masks())
             self._lazy_masks = None
         return self._save_idx
+
+    def _class_masks(self):
+        """[(class, masks)] of the last device build in class order: a class's replayed masks
+        followed by the masks of its new picks."""
+        masks, counts, classes, npicks, picks, saved_lists, _, mp = self._lazy_masks
+        h_cnt = counts.cpu().tolist()
+        out, moff = [], 0
+        for ci, c in enumerate(classes):
+            n = h_cnt[c]
+            tmp = list(saved_lists[ci])
+            mine = [p for p in picks[ci * mp:ci * mp + npicks[ci]] if p >= 0]
+            if mine:
+                idx = torch.tensor(mine, dtype=torch.int64, device=masks.device)
+                sel = masks[moff:moff + n * n].view(n, n)[idx].cpu().bool()
+                tmp.extend(sel[k].clone() for k in range(len(mine)))
+            moff += n * n
+            out.append((c, tmp))
+        return out
 
     @save_idx.setter
     def save_idx(self, value):
@@ -269,6 +269,17 @@ class MultiPrototypeReplay:
                                       ptr(out), _lib.current_stream(protos.device)),
               "repre_replay_gather")
         return out
+
+
+def _place_masks(save_idx, class_masks):
+    """The ``mask.pth`` rule of :425-452 over ``(class, masks)`` in class order: a class below
+    ``len(save_idx)`` replaces its entry, any other class is appended."""
+    for c, masks in class_masks:
+        if c < len(save_idx):
+            save_idx[c] = masks
+        else:
+            save_idx.append(masks)
+    return save_idx
 
 
 def exchange_by_class_owner(feats, labels, classes, group=None):
