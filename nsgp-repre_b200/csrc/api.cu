@@ -248,6 +248,18 @@ static size_t cov_layers_group_bytes(const ConvGeom* geoms, int n) {
          autocorr_table_bytes(ac_g.data(), (int)ac_g.size());
 }
 
+// Workspace of a staged layer: [staged operand | per-layer group table | batch-mean scratch].
+// The batch-mean scratch, or null when the layout needs none or the workspace has no room for it
+// (the staging then gathers from the input).
+static float* mean_scratch(const ConvGeom& g, float* stage, const void* workspace,
+                           size_t workspace_bytes) {
+  if (mean_scratch_elems(g) == 0) return nullptr;
+  char* m = align_up((char*)stage + stage_bytes(g) + layer_table_bytes(g), 256);
+  if (m + mean_scratch_elems(g) * sizeof(float) <= (const char*)workspace + workspace_bytes)
+    return reinterpret_cast<float*>(m);
+  return nullptr;
+}
+
 static int cov_conv2d_setup(int C, int H, int W, int kh, int kw, int sh, int sw, int ph, int pw,
                             void* workspace, size_t workspace_bytes, ConvGeom* g, float** stage) {
   NSGP_REQUIRE(make_conv_geom(C, H, W, kh, kw, sh, sw, ph, pw, g) == 0,
@@ -269,14 +281,8 @@ int nsgp_cov_conv2d_stage(const float* x, int B, int C, int H, int W, int kh, in
   float* stage;
   int rc = cov_conv2d_setup(C, H, W, kh, kw, sh, sw, ph, pw, workspace, workspace_bytes, &g, &stage);
   if (rc) return rc;
-  // [staged operand | per-layer group table | batch-mean scratch]
-  float* mean = nullptr;
-  if (mean_scratch_elems(g) > 0) {
-    char* m = align_up((char*)stage + stage_bytes(g) + layer_table_bytes(g), 256);
-    if (m + mean_scratch_elems(g) * sizeof(float) <= (char*)workspace + workspace_bytes)
-      mean = reinterpret_cast<float*>(m);
-  }
-  return launch_stage_conv(x, stage, g, B, mean, (cudaStream_t)stream_);
+  return launch_stage_conv(x, stage, g, B, mean_scratch(g, stage, workspace, workspace_bytes),
+                           (cudaStream_t)stream_);
 }
 
 int nsgp_cov_conv2d_contract(int C, int H, int W, int kh, int kw, int sh, int sw, int ph, int pw,
@@ -678,14 +684,6 @@ int nsgp_group_launch(const void* table_dev, const nsgp_group_t* group, void* st
 }
 
 // ---- grouped staging: all layer inputs of a forward in one (two) launches ----------
-static float* job_mean_scratch(const nsgp_cov_job_t& j, const ConvGeom& g, float* stage) {
-  if (mean_scratch_elems(g) == 0) return nullptr;
-  char* m = align_up((char*)stage + stage_bytes(g) + layer_table_bytes(g), 256);
-  if (m + mean_scratch_elems(g) * sizeof(float) <= (const char*)j.workspace + j.workspace_bytes)
-    return reinterpret_cast<float*>(m);
-  return nullptr;
-}
-
 size_t nsgp_cov_stage_group_bytes(const nsgp_cov_job_t* jobs, int n_jobs, int B) {
   if (!jobs || n_jobs <= 0 || B <= 0) return 1024;
   std::vector<ConvGeom> geoms;
@@ -703,7 +701,8 @@ int nsgp_cov_stage_group_build(const nsgp_cov_job_t* jobs, int n_jobs, int B,
   std::vector<float*> stages, accs, means;
   int rc = cov_jobs_setup(jobs, n_jobs, &geoms, &stages, &accs);
   if (rc) return rc;
-  for (int i = 0; i < n_jobs; ++i) means.push_back(job_mean_scratch(jobs[i], geoms[i], stages[i]));
+  for (int i = 0; i < n_jobs; ++i)
+    means.push_back(mean_scratch(geoms[i], stages[i], jobs[i].workspace, jobs[i].workspace_bytes));
   StageGroupInfo gi{};
   rc = stage_group_build(geoms.data(), stages.data(), means.data(), n_jobs, B, same_input,
                          table_dev, table_bytes, &gi, (cudaStream_t)stream_);
@@ -745,11 +744,14 @@ int nsgp_cov_stage_group_launch(void* table_dev, const nsgp_stage_group_t* sg,
                                 const nsgp_cov_job_t* jobs, const void* const* xs,
                                 void* stream_) {
   NSGP_REQUIRE(table_dev && sg && xs && jobs, "cov_stage_group_launch: null pointer");
+  const StageGroupInfo si = stage_from_abi(sg);
+  const cudaStream_t stream = (cudaStream_t)stream_;
   std::vector<ConvGeom> geoms;
-  int rc = stage_job_geoms(jobs, sg->n_jobs, &geoms);
+  int rc = stage_job_geoms(jobs, si.n_jobs, &geoms);
   if (rc) return rc;
-  return stage_group_launch(table_dev, stage_from_abi(sg), xs, (cudaStream_t)stream_,
-                            geoms.data());
+  rc = stage_group_upload(table_dev, si, xs, stream, geoms.data());
+  if (rc) return rc;
+  return stage_group_launch(table_dev, si, stream);
 }
 
 // ---- pipelined covariance pass: contraction of forward i-1 || staging of forward i ----
@@ -781,15 +783,7 @@ int nsgp_cov_pipeline_launch(const void* prev_table, const nsgp_group_t* prev_gr
       rc = group_launch(prev_table, group_from_abi(*prev_group), stream);
       if (rc) return rc;
     }
-    if (have_stage) {
-      rc = stage_group_launch_tma(stage_table, si, 0, 0, stream);
-      if (rc) return rc;
-      for (int ph = 0; ph < 2; ++ph) {
-        rc = stage_group_launch_phase(stage_table, si, ph, 0, 0, stream);
-        if (rc) return rc;
-      }
-    }
-    return 0;
+    return have_stage ? stage_group_launch(stage_table, si, stream) : 0;
   }
   // Partitioned: the sliding-window kernel (MMA-issue bound, barely affected by HBM traffic
   // next to it: +6 % measured) takes sms - stage_sms SMs, the HBM-bound first staging phase

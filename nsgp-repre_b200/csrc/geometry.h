@@ -260,13 +260,20 @@ static inline void conv_problems(const ConvGeom& g, const float* stage, float* a
 }
 constexpr int kMaxConvProblems = kAcMats;
 
+// Layouts whose vectorised staging routine reads a 16-byte aligned input itself, with no
+// batch-mean pass (plan_stage_job): flat 1x1 stride 1, and the autocorrelation layout
+static inline bool stage_flat_vec_ok(const ConvGeom& g) {
+  return g.mode == kModeFlat && g.sh == 1 && g.sw == 1 && (g.H * g.W) % 4 == 0;
+}
+static inline bool stage_ac_vec_ok(const ConvGeom& g) {
+  return g.mode == kModeAutocorr && g.W % 4 == 0 && (g.tiled || g.Ws == g.W + 4);
+}
+// per-layer staging: the routines of plan_stage_job, one launch each
 int launch_stage_conv(const float* x, float* stage, const ConvGeom& g, int B,
                       float* mean_scratch, cudaStream_t s);
 // scratch (floats) for the batch mean of the gather layouts' two-pass staging
 static inline size_t mean_scratch_elems(const ConvGeom& g) {
-  const bool vec_flat = g.mode == kModeFlat && g.sh == 1 && g.sw == 1 && (g.H * g.W) % 4 == 0;
-  const bool vec_ac = g.mode == kModeAutocorr && g.W % 4 == 0 && (g.tiled || g.Ws == g.W + 4);
-  if (vec_flat || vec_ac) return 0;
+  if (stage_flat_vec_ok(g) || stage_ac_vec_ok(g)) return 0;
   return (size_t)round_up((long long)g.C * g.H * g.W, 4);
 }
 // grouped staging (stage.cu): all layer inputs of a forward in one or two launches
@@ -309,8 +316,8 @@ size_t stage_group_bytes(const ConvGeom* geoms, int n, int B);
 int stage_group_build(const ConvGeom* geoms, float* const* stages, float* const* means, int n,
                       int B, const int* same_input, void* table_dev, size_t table_bytes,
                       StageGroupInfo* info, cudaStream_t stream);
-int stage_group_launch(const void* table_dev, const StageGroupInfo& info, const void* const* xs,
-                       cudaStream_t stream, const ConvGeom* geoms = nullptr);
+// the staging kernels of a table whose inputs stage_group_upload has set
+int stage_group_launch(const void* table_dev, const StageGroupInfo& info, cudaStream_t stream);
 int stage_group_upload(const void* table_dev, const StageGroupInfo& info, const void* const* xs,
                        cudaStream_t stream, const ConvGeom* geoms = nullptr);
 int stage_group_launch_tma(const void* table_dev, const StageGroupInfo& info, int pdl, int sms,

@@ -37,8 +37,9 @@ __device__ __forceinline__ void split_store4(float* hi, float* lo, float a, floa
 }
 
 // Every staging routine is a __device__ body over an index span (first, step, end) so that
-// the same code runs as a stand-alone grid-stride kernel (per-layer entry points) and as
-// one work item of the grouped staging kernel (stage_group_kernel, end of this file).
+// the same code runs as a stand-alone grid-stride kernel (stage_layer_kernel, per-layer entry
+// points) and as one work item of the grouped staging kernel (stage_group_kernel); both reach
+// the bodies through stage_routine.
 // I = index type: 32-bit arithmetic for the decode whenever the index space allows (a 64-bit
 // division is ~5x the instructions, and the gather routines are instruction-bound)
 template <typename I>
@@ -121,14 +122,8 @@ stage_conv_body(const float* __restrict__ x, float* __restrict__ stage, const Co
     stage_conv_body_t<long long>(x, stage, g, B, hl_stride, first, step, end);
 }
 
-__global__ void __launch_bounds__(256)
-stage_conv_kernel(const float* __restrict__ x, float* __restrict__ stage, ConvGeom g,
-                  int B, long long hl_stride) {
-  stage_conv_body(x, stage, g, B, hl_stride, blockIdx.x * (long long)blockDim.x + threadIdx.x, (long long)gridDim.x * blockDim.x, 1LL << 62);
-}
-
 // ---------------------------------------------------------------------------
-// Fast paths (same staged layout as stage_conv_kernel, 128-bit loads and stores).
+// Fast paths (same staged layout as stage_conv_body, 128-bit loads and stores).
 // ---------------------------------------------------------------------------
 // 1x1 stride-1 conv input with H*W % 4 == 0: the staged plane is the batch mean of
 // x itself.  One thread per float4.
@@ -159,13 +154,6 @@ stage_flat_vec_body(const float* __restrict__ x, float* __restrict__ stage, long
   }
 }
 
-template <int B_UNROLL>
-__global__ void __launch_bounds__(256)
-stage_flat_vec_kernel(const float* __restrict__ x, float* __restrict__ stage, long long n4,
-                      int B, long long img, long long hl_stride) {
-  stage_flat_vec_body<B_UNROLL>(x, stage, n4, B, img, hl_stride, blockIdx.x * (long long)blockDim.x + threadIdx.x, (long long)gridDim.x * blockDim.x, n4);
-}
-
 // Batch mean of x (B, n) -> out (n), n % 4 == 0, 16-byte aligned: first pass of the
 // two-pass staging used by the layouts whose second pass is a gather (stride-2 tap
 // copies, odd widths, the explicit stem): the gather then reads 1/B of the data.
@@ -193,13 +181,6 @@ batch_mean_vec_body(const float* __restrict__ x, float* __restrict__ out, long l
     *reinterpret_cast<float4*>(out + i * 4) =
         make_float4(s.x / fb, s.y / fb, s.z / fb, s.w / fb);
   }
-}
-
-template <int B_UNROLL>
-__global__ void __launch_bounds__(256)
-batch_mean_vec_kernel(const float* __restrict__ x, float* __restrict__ out, long long n4, int B,
-                      long long img) {
-  batch_mean_vec_body<B_UNROLL>(x, out, n4, B, img, blockIdx.x * (long long)blockDim.x + threadIdx.x, (long long)gridDim.x * blockDim.x, n4);
 }
 
 // 3x3 stride-1 pad-1 conv input with W % 4 == 0: each thread averages one aligned
@@ -276,13 +257,6 @@ stage_3x3s1_vec_body(const float* __restrict__ x, float* __restrict__ stage, int
   }
 }
 
-template <int B_UNROLL>
-__global__ void __launch_bounds__(256)
-stage_3x3s1_vec_kernel(const float* __restrict__ x, float* __restrict__ stage, int C, int H,
-                       int W, int B, long long hl_stride) {
-  stage_3x3s1_vec_body<B_UNROLL>(x, stage, C, H, W, B, hl_stride, blockIdx.x * (long long)blockDim.x + threadIdx.x, (long long)gridDim.x * blockDim.x, 1LL << 62);
-}
-
 // ---------------------------------------------------------------------------
 // Autocorrelation layout (3x3 s1 p1, geometry.h): three column-shifted copies of the
 // zero-extended batch mean, copy_s[c][r][x] = m~[c][r][x+s], r < H+2, x < Ws, plus the
@@ -355,13 +329,6 @@ stage_autocorr_body(const float* __restrict__ x, float* __restrict__ stage, int 
     stage_autocorr_body_t<int>(x, stage, C, H, W, Hs, Ws, B, hl_stride, tiled, rowbuf, first, step, end);
   else
     stage_autocorr_body_t<long long>(x, stage, C, H, W, Hs, Ws, B, hl_stride, tiled, rowbuf, first, step, end);
-}
-
-__global__ void __launch_bounds__(256)
-stage_autocorr_kernel(const float* __restrict__ x, float* __restrict__ stage, int C, int H,
-                      int W, int Hs, int Ws, int B, long long hl_stride, int tiled,
-                      float* __restrict__ rowbuf) {
-  stage_autocorr_body(x, stage, C, H, W, Hs, Ws, B, hl_stride, tiled, rowbuf, blockIdx.x * (long long)blockDim.x + threadIdx.x, (long long)gridDim.x * blockDim.x, 1LL << 62);
 }
 
 // W % 4 == 0, 16-byte aligned input: one thread per aligned float4 of a staged row.
@@ -450,15 +417,6 @@ stage_autocorr_vec_body(const float* __restrict__ x, float* __restrict__ stage, 
   }
 }
 
-template <int B_UNROLL>
-__global__ void __launch_bounds__(256)
-stage_autocorr_vec_kernel(const float* __restrict__ x, float* __restrict__ stage, int C, int H,
-                          int W, int B, long long hl_stride, int tiled,
-                          float* __restrict__ rowbuf) {
-  stage_autocorr_vec_body<B_UNROLL>(x, stage, C, H, W, B, hl_stride, tiled, rowbuf, blockIdx.x * (long long)blockDim.x + threadIdx.x, (long long)gridDim.x * blockDim.x,
-                                    1LL << 62);
-}
-
 // edge columns colbuf[side][shift][c][u] = m~[c][u+shift][side ? 0 : W-1] (pitch Hc) and
 // corner pixels cornerbuf[q][c][0] (pitch 4): q = 0 (H-1,W-1), 1 (H-1,0), 2 (0,W-1), 3 (0,0)
 __device__ __forceinline__ void
@@ -505,13 +463,6 @@ stage_autocorr_edges_body(const float* __restrict__ x, float* __restrict__ colbu
     dst[0] = hi;
     dst[hl_stride] = lo;
   }
-}
-
-__global__ void __launch_bounds__(256)
-stage_autocorr_edges_kernel(const float* __restrict__ x, float* __restrict__ colbuf,
-                            float* __restrict__ cornerbuf, int C, int H, int W, int Hc, int B,
-                            long long hl_stride) {
-  stage_autocorr_edges_body(x, colbuf, cornerbuf, C, H, W, Hc, B, hl_stride, blockIdx.x * (long long)blockDim.x + threadIdx.x, (long long)gridDim.x * blockDim.x, 1LL << 62);
 }
 
 // ---------------------------------------------------------------------------
@@ -625,100 +576,187 @@ stage_conv_explicit_body(const float* __restrict__ x, float* __restrict__ stage,
     stage_conv_explicit_body_t<long long>(x, stage, g, B, hl_stride, first, step, end);
 }
 
+// ---------------------------------------------------------------------------
+// Routine choice.  One planner decides which routines stage a layer, in what order, over how
+// many indices and whether each reads the input or its batch mean - for the per-layer launches
+// (launch_stage_conv, TMA off) and for the work items of a staging table (stage_job_items).
+// ---------------------------------------------------------------------------
+constexpr int kStPhaseTma = 2;         // StageRoutine::phase of the TMA kernel's routines
+constexpr int kMaxStageRoutines = 3;
+struct StageRoutine {
+  int kind;          // StageKind
+  int from_mean;     // reads the batch mean that a kStMean routine before it wrote
+  int phase;         // staging table: phase 0 / 1 of the register kernel, or kStPhaseTma
+  long long count;   // indices of the routine
+};
+
+// Fills r (in launch order) and returns the number of routines.  have_mean: the layer has
+// batch-mean scratch; aligned: x is 16-byte aligned and C*H*W % 4 == 0; tma: the TMA kernel may
+// take the routines that read the whole input.  role: 0 = plain; 1 = this flat 1x1 job also
+// writes the stride-2 subsample of a sibling job (kStFlatSub); 2 = this job is that sibling (no
+// routines of its own).
+static int plan_stage_job(const ConvGeom& g, int B, bool have_mean, bool aligned, bool tma,
+                          int role, StageRoutine* r) {
+  int n = 0;
+  auto add = [&](int phase, int kind, int from_mean, long long count) {
+    r[n++] = StageRoutine{kind, from_mean, phase, count};
+  };
+  if (role == 2) return 0;
+  const long long img = (long long)g.C * g.H * g.W;
+  const bool tma_job = tma && img % 256 == 0;
+  const int full = tma_job ? kStPhaseTma : 0;   // phase of a vectorised pass over the input
+  const int light = tma ? 1 : 0;       // light phase-0 routines ride with phase 1 under TMA
+  const bool two_pass_ok = B > 1 && aligned && have_mean;
+  if (g.mode == kModeAutocorr) {
+    if (aligned && stage_ac_vec_ok(g)) {
+      if (tma_job && g.tiled) {
+        add(kStPhaseTma, kStAcVec, 0, img / 4);   // writes the edge columns and corners too
+        return n;
+      }
+      const long long n4 = g.tiled ? (long long)ac_cblocks(g) * 128 * g.Hs * (ac_strips(g) * 8)
+                                   : (long long)g.C * g.Hs * (g.Ws / 4);
+      add(0, kStAcVec, 0, round_up(n4, 32));
+    } else {
+      const long long ns = g.tiled ? 3LL * ac_cblocks(g) * 128 * g.Hs * ac_strips(g) * 32
+                                   : (long long)g.C * g.Hs * g.Ws * 3;
+      if (two_pass_ok) {
+        add(full, kStMean, 0, img / 4);
+        add(1, kStAcScalar, 1, ns);
+      } else {
+        add(light, kStAcScalar, 0, ns);
+      }
+    }
+    add(light, kStAcEdges, 0, 6LL * g.C * ac_col_pitch(g) + 16LL * g.C);
+    return n;
+  }
+  if (aligned && stage_flat_vec_ok(g)) {
+    add(full, tma_job && role == 1 ? kStFlatSub : kStFlatVec, 0, img / 4);
+    return n;
+  }
+  if (g.mode == kModeImplicit && g.kh == 3 && g.kw == 3 && g.sh == 1 && g.sw == 1 && g.ph == 1 &&
+      g.pw == 1 && aligned && g.W % 4 == 0) {
+    add(0, kSt3x3Vec, 0, round_up((long long)g.C * g.Hs * (g.W / 4), 32));
+    return n;
+  }
+  if (tma_job && g.mode == kModeImplicit && g.kh == 3 && g.kw == 3 && g.sh == 2 && g.sw == 2 &&
+      g.ph == 1 && g.pw == 1 && g.W % 4 == 0 && g.nrowphase == 2 && g.rowphase_py[0] == 1 &&
+      g.rowphase_py[1] == 0 && g.Ht == 1) {
+    add(kStPhaseTma, kStS2x3, 0, img / 4);          // no batch-mean pass, no gather
+    return n;
+  }
+  // gather layouts: average the batch first (vectorised), then gather from the mean - unless
+  // the gather touches only a fraction of the input (strided 1x1)
+  const bool sparse = g.mode == kModeFlat && g.sh * g.sw > 1;
+  const bool two = two_pass_ok && !sparse;
+  if (two) add(full, kStMean, 0, img / 4);
+  if (g.mode == kModeExplicit)
+    add(two ? 1 : light, kStExplicit, two, (long long)g.Cs * (g.Ws / 4));
+  else
+    add(two ? 1 : light, kStConv, two, (long long)g.Cs * g.Hs * g.ncopy * (g.Ws / 4));
+  return n;
+}
+
+// The device descriptor of one staged layer (mean: its batch-mean scratch, or null)
+static StageJobDev stage_job_dev(const ConvGeom& g, float* stage, float* mean) {
+  StageJobDev j;
+  memset(&j, 0, sizeof(j));
+  j.g = g;
+  j.stage = stage;
+  j.mean = mean;
+  j.hl = stage_hl_stride(g);
+  if (g.mode == kModeAutocorr) {
+    j.rowbuf_off = ac_rowbuf_off(g);
+    j.colbuf_off = ac_colbuf_off(g);
+    j.cornerbuf_off = ac_cornerbuf_off(g);
+    j.Hc = ac_col_pitch(g);
+  }
+  return j;
+}
+
+// One routine of job j over the index span (lo + tid, step, end): the body of the per-layer
+// kernels and of every work item of stage_group_kernel.  x: the layer input (B images) or its
+// batch mean (B = 1).  row_items: the span is a work item of a staging table, which never
+// crosses an explicit im2col row (stage_job_items).
+__device__ __forceinline__ void stage_routine(int kind, const StageJobDev& j, const float* x,
+                                              int B, long long lo, int tid, long long step,
+                                              long long end, bool row_items) {
+  const ConvGeom& g = j.g;
+  const long long first = lo + tid;
+  const long long img = (long long)g.C * g.H * g.W;
+  switch (kind) {
+    case kStFlatVec:
+      stage_flat_vec_body<8>(x, j.stage, img / 4, B, img, j.hl, first, step, end);
+      break;
+    case kStAcVec:
+      stage_autocorr_vec_body<8>(x, j.stage, g.C, g.H, g.W, B, j.hl, g.tiled,
+                                 j.stage + j.rowbuf_off, first, step, end);
+      break;
+    case kStAcEdges:
+      stage_autocorr_edges_body(x, j.stage + j.colbuf_off, j.stage + j.cornerbuf_off, g.C, g.H,
+                                g.W, j.Hc, B, j.hl, first, step, end);
+      break;
+    case kStMean:
+      batch_mean_vec_body<8>(x, j.mean, img / 4, B, img, first, step, end);
+      break;
+    case kStConv:
+      stage_conv_body(x, j.stage, g, B, j.hl, first, step, end);
+      break;
+    case kStExplicit:
+      if (row_items && g.Wout % 4 == 0)
+        stage_conv_explicit_row_body(x, j.stage, g, B, j.hl, lo, tid, (int)step, end);
+      else
+        stage_conv_explicit_body(x, j.stage, g, B, j.hl, first, step, end);
+      break;
+    case kStAcScalar:
+      stage_autocorr_body(x, j.stage, g.C, g.H, g.W, g.Hs, g.Ws, B, j.hl, g.tiled,
+                          j.stage + j.rowbuf_off, first, step, end);
+      break;
+    case kSt3x3Vec:
+      stage_3x3s1_vec_body<8>(x, j.stage, g.C, g.H, g.W, B, j.hl, first, step, end);
+      break;
+    default:
+      break;
+  }
+}
+
+// Per-layer staging: one grid-stride launch per routine.  One instance per routine kind, so that
+// each compiles only its own body and keeps its own register count (stage_group_kernel, which
+// runs them all, needs 64).  The bodies stop at the end of their own index space.
+template <int KIND>
 __global__ void __launch_bounds__(256)
-stage_conv_explicit_kernel(const float* __restrict__ x, float* __restrict__ stage,
-                           ConvGeom g, int B, long long hl_stride) {
-  stage_conv_explicit_body(x, stage, g, B, hl_stride,
-                           blockIdx.x * (long long)blockDim.x + threadIdx.x,
-                           (long long)gridDim.x * blockDim.x, 1LL << 62);
+stage_layer_kernel(StageJobDev j, const float* __restrict__ x, int B) {
+  stage_routine(KIND, j, x, B, blockIdx.x * (long long)blockDim.x, threadIdx.x,
+                (long long)gridDim.x * blockDim.x, 1LL << 62, false);
 }
 
 int launch_stage_conv(const float* x, float* stage, const ConvGeom& g, int B,
                       float* mean_scratch, cudaStream_t stream) {
-  long long total = (g.mode == kModeExplicit) ? (long long)g.Cs * g.Ws
-                                              : (long long)g.Cs * g.Hs * g.Ws * g.ncopy;
-  long long hl = stage_hl_stride(g);
-  const long long img = (long long)g.C * g.H * g.W;
-  const bool aligned = (reinterpret_cast<uintptr_t>(x) & 15) == 0 && img % 4 == 0;
+  const bool aligned = (reinterpret_cast<uintptr_t>(x) & 15) == 0 &&
+                       (long long)g.C * g.H * g.W % 4 == 0;
+  StageRoutine r[kMaxStageRoutines];
+  const int n = plan_stage_job(g, B, mean_scratch != nullptr, aligned, false, 0, r);
+  const StageJobDev j = stage_job_dev(g, stage, mean_scratch);
   ProfScope prof(kProfStage, stream);
-  if (g.mode == kModeAutocorr) {
-    float* rowbuf = stage + ac_rowbuf_off(g);
-    if (aligned && g.W % 4 == 0 && (g.tiled || g.Ws == g.W + 4)) {
-      long long n = g.tiled ? (long long)ac_cblocks(g) * 128 * g.Hs * (ac_strips(g) * 8)
-                            : (long long)g.C * g.Hs * (g.Ws / 4);
-      int blocks = (int)((n + 255) / 256);
-      if (blocks > 148 * 16) blocks = 148 * 16;
-      stage_autocorr_vec_kernel<8><<<blocks, 256, 0, stream>>>(x, stage, g.C, g.H, g.W, B, hl,
-                                                              g.tiled, rowbuf);
-    } else {
-      const float* src = x;
-      int Bg = B;
-      if (B > 1 && aligned && mean_scratch != nullptr) {
-        long long n4 = img / 4;
-        int mb = (int)((n4 + 255) / 256);
-        if (mb > 148 * 16) mb = 148 * 16;
-        batch_mean_vec_kernel<8><<<mb, 256, 0, stream>>>(x, mean_scratch, n4, B, img);
-        NSGP_LAUNCHED();
-        src = mean_scratch;
-        Bg = 1;
-      }
-      long long n = g.tiled ? 3LL * ac_cblocks(g) * 128 * g.Hs * ac_strips(g) * 32
-                            : (long long)g.C * g.Hs * g.Ws * 3;
-      int blocks = (int)((n + 255) / 256);
-      if (blocks > 148 * 32) blocks = 148 * 32;
-      stage_autocorr_kernel<<<blocks, 256, 0, stream>>>(src, stage, g.C, g.H, g.W, g.Hs, g.Ws, Bg,
-                                                       hl, g.tiled, rowbuf);
+  for (int k = 0; k < n; ++k) {
+    void (*kernel)(StageJobDev, const float*, int) = nullptr;
+    int per_sm = 16;                               // blocks per SM at most
+    switch (r[k].kind) {
+      case kStFlatVec: kernel = stage_layer_kernel<kStFlatVec>; break;
+      case kStAcVec: kernel = stage_layer_kernel<kStAcVec>; break;
+      case kStMean: kernel = stage_layer_kernel<kStMean>; break;
+      case kSt3x3Vec: kernel = stage_layer_kernel<kSt3x3Vec>; break;
+      case kStAcEdges: kernel = stage_layer_kernel<kStAcEdges>; per_sm = 8; break;
+      case kStAcScalar: kernel = stage_layer_kernel<kStAcScalar>; per_sm = 32; break;
+      case kStConv: kernel = stage_layer_kernel<kStConv>; per_sm = 32; break;
+      case kStExplicit: kernel = stage_layer_kernel<kStExplicit>; per_sm = 32; break;
+      default: break;
     }
+    NSGP_REQUIRE(kernel != nullptr, "stage: routine %d has no per-layer kernel", r[k].kind);
+    const int blocks = (int)std::min((r[k].count + 255) / 256, 148LL * per_sm);
+    kernel<<<blocks, 256, 0, stream>>>(j, r[k].from_mean ? mean_scratch : x,
+                                       r[k].from_mean ? 1 : B);
     NSGP_LAUNCHED();
-    const int Hc = ac_col_pitch(g);
-    long long ne = 6LL * g.C * Hc + 16LL * g.C;
-    int eb = (int)((ne + 255) / 256);
-    if (eb > 148 * 8) eb = 148 * 8;
-    stage_autocorr_edges_kernel<<<eb, 256, 0, stream>>>(x, stage + ac_colbuf_off(g),
-                                                        stage + ac_cornerbuf_off(g), g.C, g.H,
-                                                        g.W, Hc, B, hl);
-    NSGP_LAUNCHED();
-    return 0;
   }
-  if (g.mode == kModeFlat && g.sh == 1 && g.sw == 1 && aligned && (g.H * g.W) % 4 == 0) {
-    long long n4 = (long long)g.C * g.H * g.W / 4;
-    int blocks = (int)((n4 + 255) / 256);
-    if (blocks > 148 * 16) blocks = 148 * 16;
-    stage_flat_vec_kernel<8><<<blocks, 256, 0, stream>>>(x, stage, n4, B, img, hl);
-  } else if (g.mode == kModeImplicit && g.kh == 3 && g.kw == 3 && g.sh == 1 && g.sw == 1 &&
-             g.ph == 1 && g.pw == 1 && aligned && g.W % 4 == 0) {
-    long long n = (long long)g.C * g.Hs * (g.W / 4);
-    int blocks = (int)((n + 255) / 256);
-    if (blocks > 148 * 16) blocks = 148 * 16;
-    stage_3x3s1_vec_kernel<8><<<blocks, 256, 0, stream>>>(x, stage, g.C, g.H, g.W, B, hl);
-  } else {
-    // gather layouts: average the batch first (vectorised), then gather from the mean -
-    // unless the gather touches only a fraction of the input (strided 1x1)
-    const float* src = x;
-    int Bg = B;
-    const bool sparse = g.mode == kModeFlat && g.sh * g.sw > 1;
-    if (B > 1 && aligned && mean_scratch != nullptr && !sparse) {
-      long long n4 = img / 4;
-      int mb = (int)((n4 + 255) / 256);
-      if (mb > 148 * 16) mb = 148 * 16;
-      batch_mean_vec_kernel<8><<<mb, 256, 0, stream>>>(x, mean_scratch, n4, B, img);
-      NSGP_LAUNCHED();
-      src = mean_scratch;
-      Bg = 1;
-    }
-    if (g.mode == kModeExplicit) {
-      long long ne = (long long)g.Cs * (g.Ws / 4);
-      int grid = (int)((ne + 255) / 256);
-      if (grid > 148 * 32) grid = 148 * 32;
-      stage_conv_explicit_kernel<<<grid, 256, 0, stream>>>(src, stage, g, Bg, hl);
-    } else {
-      int blocks = (int)((total / 4 + 255) / 256);
-      if (blocks > 148 * 32) blocks = 148 * 32;
-      if (blocks < 1) blocks = 1;
-      stage_conv_kernel<<<blocks, 256, 0, stream>>>(src, stage, g, Bg, hl);
-    }
-  }
-  NSGP_LAUNCHED();
   return 0;
 }
 
@@ -742,46 +780,8 @@ stage_group_kernel(const StageJobDev* __restrict__ jobs, const StageItem* __rest
   for (int w = blockIdx.x; w < n_items; w += gridDim.x) {
     const StageItem it = items[w];
     const StageJobDev& j = jobs[it.job];
-    const ConvGeom& g = j.g;
-    const float* x = it.from_mean ? j.mean : xs[it.job];
-    const int Bx = it.from_mean ? 1 : B;
-    const long long first = it.lo + threadIdx.x, step = blockDim.x, end = it.hi;
-    const long long img = (long long)g.C * g.H * g.W;
-    switch (it.kind) {
-      case kStFlatVec:
-        stage_flat_vec_body<8>(x, j.stage, img / 4, Bx, img, j.hl, first, step, end);
-        break;
-      case kStAcVec:
-        stage_autocorr_vec_body<8>(x, j.stage, g.C, g.H, g.W, Bx, j.hl, g.tiled,
-                                   j.stage + j.rowbuf_off, first, step, end);
-        break;
-      case kStAcEdges:
-        stage_autocorr_edges_body(x, j.stage + j.colbuf_off, j.stage + j.cornerbuf_off, g.C,
-                                  g.H, g.W, j.Hc, Bx, j.hl, first, step, end);
-        break;
-      case kStMean:
-        batch_mean_vec_body<8>(x, j.mean, img / 4, Bx, img, first, step, end);
-        break;
-      case kStConv:
-        stage_conv_body(x, j.stage, g, Bx, j.hl, first, step, end);
-        break;
-      case kStExplicit:
-        if (g.Wout % 4 == 0)                        // items are row-aligned (plan_stage_job)
-          stage_conv_explicit_row_body(x, j.stage, g, Bx, j.hl, it.lo, threadIdx.x, blockDim.x,
-                                       end);
-        else
-          stage_conv_explicit_body(x, j.stage, g, Bx, j.hl, first, step, end);
-        break;
-      case kStAcScalar:
-        stage_autocorr_body(x, j.stage, g.C, g.H, g.W, g.Hs, g.Ws, Bx, j.hl, g.tiled,
-                            j.stage + j.rowbuf_off, first, step, end);
-        break;
-      case kSt3x3Vec:
-        stage_3x3s1_vec_body<8>(x, j.stage, g.C, g.H, g.W, Bx, j.hl, first, step, end);
-        break;
-      default:
-        break;
-    }
+    stage_routine(it.kind, j, it.from_mean ? j.mean : xs[it.job], it.from_mean ? 1 : B, it.lo,
+                  threadIdx.x, blockDim.x, it.hi, true);
   }
   tl_end(tl);
 }
@@ -1256,100 +1256,35 @@ stage_tma_kernel(const StageJobDev* __restrict__ jobs, const StageItem* __restri
   tl_end(tl);
 }
 
-// Plans one layer: the same routine choice as launch_stage_conv (x assumed 16-byte aligned;
-// the caller checks).  Appends to items[list] when items != nullptr, always counts.
-// lists: [0] phase 0, register kernel; [1] phase 1 (after the batch means; also the light
-// phase-0 routines when the TMA kernel takes the heavy ones); [2] phase 0, TMA kernel
 static bool stage_tma_enabled(int B) {
   return tma_box_rows(B) > 0 && tma_ring_stages(B) >= kTmaGroups;
 }
 
-// role: 0 = plain; 1 = this flat 1x1 job also writes the stride-2 subsample of a sibling job
-// (kStFlatSub); 2 = this job is that sibling (no items of its own)
-static bool stage_sub_pair_ok(const ConvGeom& sub, const ConvGeom& full, int B);
-static void plan_stage_job(const ConvGeom& g, int job, int B, bool have_mean,
-                           std::vector<StageItem>* items /* [3] or null */, size_t* counts,
-                           int role = 0) {
-  if (role == 2) return;
-  const long long img = (long long)g.C * g.H * g.W;
-  const bool aligned = img % 4 == 0;
-  const bool tma = stage_tma_enabled(B);
-  const bool tma_job = tma && img % 256 == 0;
-  auto add = [&](int list, int kind, int from_mean, long long total, long long chunk) {
-    for (long long lo = 0; lo < total; lo += chunk) {
-      ++counts[list];
-      if (items) {
+// The work items of one job of a staging table (inputs 16-byte aligned: stage_group_upload),
+// appended to items[phase] when items != nullptr; returns their number.  An item spans 32 TMA
+// stages, 2048 vector or 8192 scalar indices, and never crosses an explicit im2col row
+// (stage_conv_explicit_row_body).
+static size_t stage_job_items(const ConvGeom& g, int job, int B, bool have_mean, int role,
+                              std::vector<StageItem>* items /* [3] or null */) {
+  StageRoutine r[kMaxStageRoutines];
+  const bool aligned = (long long)g.C * g.H * g.W % 4 == 0;
+  const int n = plan_stage_job(g, B, have_mean, aligned, stage_tma_enabled(B), role, r);
+  size_t count = 0;
+  for (int k = 0; k < n; ++k) {
+    const long long chunk = r[k].phase == kStPhaseTma ? 32LL * 64 * tma_box_rows(B)
+                            : r[k].kind == kStAcScalar ? 8192 : 2048;
+    const long long span = r[k].kind == kStExplicit ? g.Ws / 4 : r[k].count;
+    for (long long base = 0; base < r[k].count; base += span)
+      for (long long lo = 0; lo < span; lo += chunk, ++count) {
+        if (!items) continue;
         StageItem it{};
-        it.job = job; it.kind = (short)kind; it.from_mean = (short)from_mean;
-        it.lo = lo; it.hi = lo + chunk < total ? lo + chunk : total;
-        items[list].push_back(it);
+        it.job = job; it.kind = (short)r[k].kind; it.from_mean = (short)r[k].from_mean;
+        it.lo = base + lo;
+        it.hi = base + (lo + chunk < span ? lo + chunk : span);
+        items[r[k].phase].push_back(it);
       }
-    }
-  };
-  const long long kVec = 2048, kScalar = 8192;
-  const long long kTma = 32LL * 64 * (tma ? tma_box_rows(B) : 1);    // 32 stages per item
-  const int light = tma ? 1 : 0;       // light phase-0 routines ride with phase 1 under TMA
-  const bool two_pass_ok = B > 1 && aligned && have_mean;
-  if (g.mode == kModeAutocorr) {
-    if (aligned && g.W % 4 == 0 && (g.tiled || g.Ws == g.W + 4)) {
-      if (tma_job && g.tiled) {
-        add(2, kStAcVec, 0, img / 4, kTma);      // writes the edge columns and corners too
-        return;
-      } else {
-        const long long n = g.tiled ? (long long)ac_cblocks(g) * 128 * g.Hs * (ac_strips(g) * 8)
-                                    : (long long)g.C * g.Hs * (g.Ws / 4);
-        add(0, kStAcVec, 0, round_up(n, 32), kVec);
-      }
-    } else {
-      const long long n = g.tiled ? 3LL * ac_cblocks(g) * 128 * g.Hs * ac_strips(g) * 32
-                                  : (long long)g.C * g.Hs * g.Ws * 3;
-      if (two_pass_ok) {
-        if (tma_job) add(2, kStMean, 0, img / 4, kTma); else add(0, kStMean, 0, img / 4, kVec);
-        add(1, kStAcScalar, 1, n, kScalar);
-      } else {
-        add(light, kStAcScalar, 0, n, kScalar);
-      }
-    }
-    add(light, kStAcEdges, 0, 6LL * g.C * ac_col_pitch(g) + 16LL * g.C, kVec);
-    return;
   }
-  if (g.mode == kModeFlat && g.sh == 1 && g.sw == 1 && aligned && (g.H * g.W) % 4 == 0) {
-    if (tma_job) add(2, role == 1 ? kStFlatSub : kStFlatVec, 0, img / 4, kTma);
-    else add(0, kStFlatVec, 0, img / 4, kVec);
-    return;
-  }
-  if (g.mode == kModeImplicit && g.kh == 3 && g.kw == 3 && g.sh == 1 && g.sw == 1 && g.ph == 1 &&
-      g.pw == 1 && aligned && g.W % 4 == 0) {
-    add(0, kSt3x3Vec, 0, round_up((long long)g.C * g.Hs * (g.W / 4), 32), kVec);
-    return;
-  }
-  if (tma_job && g.mode == kModeImplicit && g.kh == 3 && g.kw == 3 && g.sh == 2 && g.sw == 2 &&
-      g.ph == 1 && g.pw == 1 && g.W % 4 == 0 && g.nrowphase == 2 && g.rowphase_py[0] == 1 &&
-      g.rowphase_py[1] == 0 && g.Ht == 1) {
-    add(2, kStS2x3, 0, img / 4, kTma);              // no batch-mean pass, no gather
-    return;
-  }
-  const bool sparse = g.mode == kModeFlat && g.sh * g.sw > 1;
-  const bool two = two_pass_ok && !sparse;
-  if (two) {
-    if (tma_job) add(2, kStMean, 0, img / 4, kTma); else add(0, kStMean, 0, img / 4, kVec);
-  }
-  if (g.mode == kModeExplicit) {
-    // one item never crosses an im2col row (stage_conv_explicit_row_body)
-    const long long w4 = g.Ws / 4;
-    for (int row = 0; row < g.Cs; ++row)
-      for (long long lo = 0; lo < w4; lo += kVec) {
-        ++counts[two ? 1 : light];
-        if (items) {
-          StageItem it{};
-          it.job = job; it.kind = (short)kStExplicit; it.from_mean = (short)(two ? 1 : 0);
-          it.lo = row * w4 + lo;
-          it.hi = row * w4 + (lo + kVec < w4 ? lo + kVec : w4);
-          items[two ? 1 : light].push_back(it);
-        }
-      }
-  } else
-    add(two ? 1 : light, kStConv, two ? 1 : 0, (long long)g.Cs * g.Hs * g.ncopy * (g.Ws / 4), kVec);
+  return count;
 }
 
 namespace tc { int sm_count(); }
@@ -1366,9 +1301,9 @@ static bool stage_sub_pair_ok(const ConvGeom& sub, const ConvGeom& full, int B) 
 }
 
 size_t stage_group_bytes(const ConvGeom* geoms, int n, int B) {
-  size_t counts[3] = {0, 0, 0};
-  for (int i = 0; i < n; ++i) plan_stage_job(geoms[i], i, B, true, nullptr, counts);
-  return (size_t)n * sizeof(StageJobDev) + (counts[0] + counts[1] + counts[2]) * sizeof(StageItem) +
+  size_t n_items = 0;
+  for (int i = 0; i < n; ++i) n_items += stage_job_items(geoms[i], i, B, true, 0, nullptr);
+  return (size_t)n * sizeof(StageJobDev) + n_items * sizeof(StageItem) +
          (size_t)n * sizeof(void*) + (size_t)n * sizeof(CUtensorMap) + 2048;
 }
 
@@ -1388,7 +1323,6 @@ int stage_group_build(const ConvGeom* geoms, float* const* stages, float* const*
   }
   std::vector<StageJobDev> jobs(n);
   std::vector<StageItem> items[3];
-  size_t counts[3] = {0, 0, 0};
   // pairs (1x1 s2 job, 1x1 s1 job on the same tensor): role[i] = 2, role[k] = 1, sub_of[k] = i
   std::vector<int> role(n, 0), sub_of(n, -1);
   for (int i = 0; i < n && same_input; ++i) {
@@ -1399,17 +1333,7 @@ int stage_group_build(const ConvGeom* geoms, float* const* stages, float* const*
   for (int i = 0; i < n; ++i) {
     const ConvGeom& g = geoms[i];
     StageJobDev& j = jobs[i];
-    memset(&j, 0, sizeof(j));
-    j.g = g;
-    j.stage = stages[i];
-    j.mean = means[i];
-    j.hl = stage_hl_stride(g);
-    if (g.mode == kModeAutocorr) {
-      j.rowbuf_off = ac_rowbuf_off(g);
-      j.colbuf_off = ac_colbuf_off(g);
-      j.cornerbuf_off = ac_cornerbuf_off(g);
-      j.Hc = ac_col_pitch(g);
-    }
+    j = stage_job_dev(g, stages[i], means[i]);
     if (role[i] == 1) {
       const ConvGeom& sg = geoms[sub_of[i]];
       j.sub_stage = stages[sub_of[i]];
@@ -1420,7 +1344,7 @@ int stage_group_build(const ConvGeom* geoms, float* const* stages, float* const*
       NSGP_CHECK_CUDA(cudaMemsetAsync(stages[sub_of[i]], 0, stage_bytes(sg), stream));
     }
     const size_t before = items[2].size();
-    plan_stage_job(g, i, B, means[i] != nullptr, items, counts, role[i]);
+    stage_job_items(g, i, B, means[i] != nullptr, role[i], items);
     // the TMA autocorrelation / stride-2 routines write the data words only: the padding of
     // the layouts (halo rows, columns past the row end, channels >= C) is zeroed here, once
     // per table
@@ -1580,17 +1504,11 @@ int stage_group_launch_phase(const void* table_dev, const StageGroupInfo& info, 
   return 0;
 }
 
-int stage_group_launch(const void* table_dev, const StageGroupInfo& info, const void* const* xs,
-                       cudaStream_t stream, const ConvGeom* geoms) {
-  int rc = stage_group_upload(table_dev, info, xs, stream, geoms);
-  if (rc) return rc;
-  rc = stage_group_launch_tma(table_dev, info, 0, 0, stream);
-  if (rc) return rc;
-  for (int ph = 0; ph < 2; ++ph) {
+int stage_group_launch(const void* table_dev, const StageGroupInfo& info, cudaStream_t stream) {
+  int rc = stage_group_launch_tma(table_dev, info, 0, 0, stream);
+  for (int ph = 0; ph < 2 && rc == 0; ++ph)
     rc = stage_group_launch_phase(table_dev, info, ph, 0, 0, stream);
-    if (rc) return rc;
-  }
-  return 0;
+  return rc;
 }
 
 // ---------------------------------------------------------------------------

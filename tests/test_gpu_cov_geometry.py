@@ -151,9 +151,9 @@ def _cases():
 
 
 # ---------------------------------------------------- restated layout and routine choice
-# Mirrors make_conv_geom (geometry.h: the layout), plan_stage_job (stage.cu: the routines of
-# deferred mode's staging table) and launch_stage_conv (stage.cu: grouped and immediate modes,
-# and the per-layer fallback of deferred mode).  Change them together.
+# Mirrors make_conv_geom (geometry.h: the layout) and plan_stage_job (stage.cu: the routines that
+# stage a layer, for deferred mode's staging table and for the per-layer launches of grouped and
+# immediate modes and of deferred mode's fallback).  Change them together.
 def _layout(C, H, W, kh, kw, sh, sw, ph, pw):
     if (kh, kw, sh, sw, ph, pw) == (3, 3, 1, 1, 1, 1) and C % 8 == 0 and H >= 3 and W >= 3:
         return "autocorr"
@@ -179,80 +179,72 @@ def _sub_pair_ok(sub, full, B):
             sub[5:7] == (2, 2) and sub[:3] == full[:3] and ((W - 1) // 2 + 1) * 2 == W)
 
 
-def _routine(geom, B, planner, aligned=True, paired=False):
-    """Routines that stage one layer: planner "plan" (plan_stage_job; the caller checked that the
-    input is 16-byte aligned) or "launch" (launch_stage_conv; ``aligned``: x % 16 == 0)."""
+def _routine(geom, B, tma, aligned, paired=False):
+    """Routines that stage one layer (plan_stage_job).  ``tma``: the TMA kernel may take the layer
+    (staging tables); ``aligned``: x % 16 == 0 (staging tables require it)."""
     C, H, W, kh, kw, sh, sw, ph, pw = geom
     mode = _layout(*geom)
-    Wout = (W + 2 * pw - kw) // sw + 1
     img = C * H * W
     aligned = aligned and img % 4 == 0
-    vec_flat = mode == "flat" and (sh, sw) == (1, 1) and H * W % 4 == 0
-    s1x3 = (kh, kw, sh, sw, ph, pw) == (3, 3, 1, 1, 1, 1)
-    sparse = mode == "flat" and sh * sw > 1
-    if planner == "plan":
-        tma = _tma_enabled(B) and img % 256 == 0
-        mean = ("Mean/tma",) if tma else ("Mean",)
-        two = B > 1 and aligned             # mean_scratch exists wherever a routine reads it
-        if mode == "autocorr":
-            if aligned and W % 4 == 0:
-                return ("AcVec/tma",) if tma else ("AcVec", "AcEdges")
-            return (mean if two else ()) + ("AcScalar", "AcEdges")
-        if vec_flat and aligned:
-            if tma:
-                return ("FlatSub/tma",) if paired else ("FlatVec/tma",)
-            return ("FlatVec",)
-        if mode == "implicit" and s1x3 and aligned and W % 4 == 0:
-            return ("3x3Vec",)
-        if tma and mode == "implicit" and (kh, kw, sh, sw, ph, pw) == (3, 3, 2, 2, 1, 1) and \
-                W % 4 == 0:
-            return ("S2x3/tma",)
-        two = two and not sparse
-        body = ("Explicit/rows" if Wout % 4 == 0 else "Explicit") if mode == "explicit" else "Conv"
-        return (mean if two else ()) + (body,)
+    tma_job = tma and img % 256 == 0
+    full = "/tma" if tma_job else ""     # a vectorised pass over the whole input
+    two = B > 1 and aligned              # mean_scratch exists wherever a routine reads it
     if mode == "autocorr":
         if aligned and W % 4 == 0:
-            return ("AcVec", "AcEdges")
-        return (("Mean",) if B > 1 and aligned else ()) + ("AcScalar", "AcEdges")
-    if vec_flat and aligned:
-        return ("FlatVec",)
-    if mode == "implicit" and s1x3 and aligned and W % 4 == 0:
+            return ("AcVec/tma",) if tma_job else ("AcVec", "AcEdges")
+        return (("Mean" + full,) if two else ()) + ("AcScalar", "AcEdges")
+    if mode == "flat" and (sh, sw) == (1, 1) and H * W % 4 == 0 and aligned:
+        return ("FlatSub/tma",) if tma_job and paired else ("FlatVec" + full,)
+    if mode == "implicit" and (kh, kw, sh, sw, ph, pw) == (3, 3, 1, 1, 1, 1) and aligned and \
+            W % 4 == 0:
         return ("3x3Vec",)
-    return (("Mean",) if B > 1 and aligned and not sparse else ()) + \
-        ("Explicit" if mode == "explicit" else "Conv",)
+    if tma_job and mode == "implicit" and (kh, kw, sh, sw, ph, pw) == (3, 3, 2, 2, 1, 1) and \
+            W % 4 == 0:
+        return ("S2x3/tma",)
+    two = two and not (mode == "flat" and sh * sw > 1)
+    return (("Mean" + full,) if two else ()) + ("Explicit" if mode == "explicit" else "Conv",)
 
 
-# every routine sequence the two planners can pick, with the batch classes the tests must reach
-# it with ("1": B = 1, "+": some B > 1)
+def _table_routine(geom, B, paired=False):
+    """Routines of a layer's staging-table items.  The items of explicit im2col never cross an
+    im2col row, and stage_routine stages them row by row when Wout % 4 == 0 ("Explicit/rows")."""
+    C, H, W, kh, kw, sh, sw, ph, pw = geom
+    Wout = (W + 2 * pw - kw) // sw + 1
+    return tuple("Explicit/rows" if r == "Explicit" and Wout % 4 == 0 else r
+                 for r in _routine(geom, B, _tma_enabled(B), True, paired))
+
+
+# every routine sequence of the staging table and of the per-layer launches, with the batch
+# classes the tests must reach it with ("1": B = 1, "+": some B > 1)
 EXPECTED_ROUTES = {
-    ("plan", ("AcVec/tma",)): "1+",
-    ("plan", ("AcVec", "AcEdges")): "1+",
-    ("plan", ("Mean/tma", "AcScalar", "AcEdges")): "+",
-    ("plan", ("Mean", "AcScalar", "AcEdges")): "+",
-    ("plan", ("AcScalar", "AcEdges")): "1",     # C % 8 = 0: B > 1 always has the batch mean
-    ("plan", ("FlatVec/tma",)): "1+",
-    ("plan", ("FlatSub/tma",)): "1+",
-    ("plan", ("FlatVec",)): "1+",
-    ("plan", ("3x3Vec",)): "1+",
-    ("plan", ("S2x3/tma",)): "1+",
-    ("plan", ("Conv",)): "1+",                  # B > 1: strided 1x1
-    ("plan", ("Mean/tma", "Conv")): "+",
-    ("plan", ("Mean", "Conv")): "+",
-    ("plan", ("Explicit/rows",)): "1+",         # B > 1: C*H*W % 4 != 0
-    ("plan", ("Explicit",)): "1+",
-    ("plan", ("Mean/tma", "Explicit/rows")): "+",
-    ("plan", ("Mean", "Explicit/rows")): "+",
-    ("plan", ("Mean/tma", "Explicit")): "+",
-    ("plan", ("Mean", "Explicit")): "+",
-    ("launch", ("AcVec", "AcEdges")): "1+",
-    ("launch", ("Mean", "AcScalar", "AcEdges")): "+",
-    ("launch", ("AcScalar", "AcEdges")): "1+",  # B > 1: misaligned input
-    ("launch", ("FlatVec",)): "1+",
-    ("launch", ("3x3Vec",)): "1+",
-    ("launch", ("Conv",)): "1+",
-    ("launch", ("Mean", "Conv")): "+",
-    ("launch", ("Explicit",)): "1+",
-    ("launch", ("Mean", "Explicit")): "+",
+    ("table", ("AcVec/tma",)): "1+",
+    ("table", ("AcVec", "AcEdges")): "1+",
+    ("table", ("Mean/tma", "AcScalar", "AcEdges")): "+",
+    ("table", ("Mean", "AcScalar", "AcEdges")): "+",
+    ("table", ("AcScalar", "AcEdges")): "1",    # C % 8 = 0: B > 1 always has the batch mean
+    ("table", ("FlatVec/tma",)): "1+",
+    ("table", ("FlatSub/tma",)): "1+",
+    ("table", ("FlatVec",)): "1+",
+    ("table", ("3x3Vec",)): "1+",
+    ("table", ("S2x3/tma",)): "1+",
+    ("table", ("Conv",)): "1+",                 # B > 1: strided 1x1
+    ("table", ("Mean/tma", "Conv")): "+",
+    ("table", ("Mean", "Conv")): "+",
+    ("table", ("Explicit/rows",)): "1+",        # B > 1: C*H*W % 4 != 0
+    ("table", ("Explicit",)): "1+",
+    ("table", ("Mean/tma", "Explicit/rows")): "+",
+    ("table", ("Mean", "Explicit/rows")): "+",
+    ("table", ("Mean/tma", "Explicit")): "+",
+    ("table", ("Mean", "Explicit")): "+",
+    ("layer", ("AcVec", "AcEdges")): "1+",
+    ("layer", ("Mean", "AcScalar", "AcEdges")): "+",
+    ("layer", ("AcScalar", "AcEdges")): "1+",   # B > 1: misaligned input
+    ("layer", ("FlatVec",)): "1+",
+    ("layer", ("3x3Vec",)): "1+",
+    ("layer", ("Conv",)): "1+",
+    ("layer", ("Mean", "Conv")): "+",
+    ("layer", ("Explicit",)): "1+",
+    ("layer", ("Mean", "Explicit")): "+",
 }
 
 
@@ -695,17 +687,18 @@ def test_one_key_several_extents_narrow_map(pkg, mode):
 
 # ------------------------------------------------------------- 5. routes (no GPU)
 def _route_cases():
-    """(planner, geometry, B, aligned, paired) of every staged layer the GPU tests above run."""
+    """(route, geometry, B, aligned, paired) of every staged layer the GPU tests above run: route
+    "table" (deferred mode's staging table) or "layer" (the per-layer launches)."""
     out = []
     for geom, Bs, _det in GRID:
         for B in Bs:
-            out += [("plan", geom, B, True, False), ("launch", geom, B, True, False),
-                    ("plan", COMPANION, B, True, False), ("launch", COMPANION, B, True, False)]
+            out += [("table", geom, B, True, False), ("layer", geom, B, True, False),
+                    ("table", COMPANION, B, True, False), ("layer", COMPANION, B, True, False)]
     for geom in MISALIGNED:
         for B in MISALIGNED_BS:
-            out.append(("launch", geom, B, False, False))    # also deferred mode's fallback
+            out.append(("layer", geom, B, False, False))     # also deferred mode's fallback
     for geom in RAGGED:
-        out += [("launch", geom, 3, True, False), ("launch", geom, 1, True, False)]
+        out += [("layer", geom, 3, True, False), ("layer", geom, 1, True, False)]
     for _name, layers, order in PAIRS:
         for B in (1, 2):
             full = [g for g in layers.values() if g[5:7] == (1, 1)]
@@ -714,19 +707,20 @@ def _route_cases():
                     _sub_pair_ok(s, g, B) for s in layers.values() if s[5:7] == (2, 2))
                 sibling = g[5:7] == (2, 2) and full and _sub_pair_ok(g, full[0], B)
                 if not sibling:
-                    out.append(("plan", g, B, True, paired))
-                out.append(("launch", g, B, True, False))
+                    out.append(("table", g, B, True, paired))
+                out.append(("layer", g, B, True, False))
     return out
 
 
 def test_every_staging_route_is_reached():
     """The layer geometries, batch sizes and input alignments of this file reach every routine
-    sequence that plan_stage_job and launch_stage_conv can pick, each with B = 1 and with some
-    B > 1 where the planner allows it (EXPECTED_ROUTES)."""
+    sequence that plan_stage_job can pick for a staging table and for the per-layer launches,
+    each with B = 1 and with some B > 1 where the planner allows it (EXPECTED_ROUTES)."""
     reached = {}
-    for planner, geom, B, aligned, paired in _route_cases():
-        key = (planner, _routine(geom, B, planner, aligned, paired))
-        reached.setdefault(key, set()).add("1" if B == 1 else "+")
+    for route, geom, B, aligned, paired in _route_cases():
+        seq = _table_routine(geom, B, paired) if route == "table" else \
+            _routine(geom, B, tma=False, aligned=aligned)
+        reached.setdefault((route, seq), set()).add("1" if B == 1 else "+")
     unknown = set(reached) - set(EXPECTED_ROUTES)
     assert not unknown, unknown
     missing = {k: v for k, v in EXPECTED_ROUTES.items() if not set(v) <= reached.get(k, set())}
